@@ -18,6 +18,9 @@ ciphertexts under the private key (full VerifyDecrypt witness).
 
 `--impl reference` times that CPU restatement alone (node does not exist in this image, so the
 reference's own JavaScript cannot run; see DESIGN.md).
+
+`--dump-outputs DIR` writes the arrays the last timed step returned (a seeded sample of 4096 rows of each) to
+DIR/<name>.npy, so that two builds of the engine can be compared on identical inputs.
 """
 from __future__ import annotations
 
@@ -42,6 +45,26 @@ WORKLOAD = "NTRU-HPS N=509 q=2048 p=3, {rows} ciphertexts under one key per GPU,
 def load_key():
     g = dict(np.load(os.path.join(ROOT, "tests", "golden", f"{CONFIG}.npz")))
     return g
+
+
+DUMP_ROWS = 4096     # rows of each output written by --dump-outputs: 6 arrays x (6 N + 4) float32 columns = 50 MB at N = 509
+
+
+def dump_outputs(dirname, arrays):
+    """Writes the same seeded sample of rows of every array in `arrays` (name -> device tensor of shape (B, width)) to
+    dirname/<name>.npy as float32 (exact: every value is below 2^16).  The sample depends on B alone, and the bench's
+    inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+    import torch
+    B = next(iter(arrays.values())).shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_ROWS), replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        x = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy()
+        if x.dtype == np.int16:
+            x = x.view(np.uint16)      # the ABI's uint16 coefficients travel in int16 tensors
+        np.save(os.path.join(dirname, f"{name}.npy"), x.astype(np.float32))
+    return {"dir": dirname, "rows": len(rows),
+            "row_sample": "numpy default_rng(0).choice(rows_per_gpu, min(rows_per_gpu, 4096), replace=False), sorted; rank 0"}
 
 
 def peaks():
@@ -512,6 +535,12 @@ def run_ours(args, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value_cts = world * B * args.steps / (ms * 1e-3)
+    # what the last timed step computed, as the host-buffer ABI returns it (remainderE == value, remainder2 == plaintext)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, {
+            "value": value[:, :N], "quotientE": quo[:, :N + 1], "plaintext": out[:, :N],
+            "quotient1": q1[:, :N + 1], "remainder1": r1[:, :N + 1], "quotient2": q2[:, :N + 1]})
 
     # ---- secondary figures (outside the timed region above): value-only mode, encrypt-only, decrypt-only ----
     def timed_ms(fn, iters=5):
@@ -705,6 +734,8 @@ def run_ours(args, rank, world, local_rank):
         "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "extras": extras,
     }
     extras["configs"] = configs
+    if dumped:
+        line["dump_outputs"] = dumped
     if not args.no_cpu and world == 1:                  # the CPU leg runs at N = 1 only (rank 0's host cores)
         line["cpu_baseline"] = cpu_baseline(g)
     print(json.dumps(line), flush=True)
@@ -724,7 +755,14 @@ def main():
     ap.add_argument("--path", type=int, default=0, help="0 auto, 1 fp32 CUDA-core schedule, 2 tcgen05 schedule, 3 register-fragment IMMA schedule")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--configs", default="c1,c3,c4,c5", help="other BASELINE configs to run after the headline (extras.configs); '' for none")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of 4096 rows of every output of the last step to DIR/<name>.npy "
+                         "(float32, 50 MB; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
