@@ -91,7 +91,8 @@ enum {
   NTRU_K_DEC_IMMA = 8,      /* mma.sync (IMMA) decrypt (both products) */
   NTRU_K_MULDIV = 9,        /* mma.sync (IMMA) multiply + divide by 1 - x^N (verifyKeysInputs products) */
   NTRU_K_PACK = 10,         /* packOutput / unpackInput bit packing */
-  NTRU_K_COUNT = 11
+  NTRU_K_INVERSE = 11,      /* key generation: f^-1 modulo 2 and modulo 3 (divsteps) */
+  NTRU_K_COUNT = 12
 };
 
 /* new NTRU({N,p,q}) -- index.js:8-28.  p must be 3, q a power of two in [4, 8192], 8 <= N <= 1024
@@ -169,10 +170,12 @@ int ntru_muldiv_dev(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int
 
 /* loadPrivateKeyF + generatePublicKeyH for B keys at once -- index.js:30-79, 491-514.  f, g: B x N ternary (the
  * generateCustomArray draws stay with the caller's CSPRNG).  fp = f^-1 mod (p, x^N-1), fq = f^-1 mod (q, x^N-1),
- * h = (p fq) * g mod (q, x^N-1); rows of N entries, un-trimmed.  The extended-Euclid inversions modulo 2 and modulo p
- * run on the host (sequential, index.js:425-459); the Newton lifting 2 -> q (index.js:497-509) and h run on the GPU.
- * valid[b] = 1 iff f_b is invertible modulo 2 and modulo p -- then the outputs equal the reference's (the inverse is
- * unique); otherwise the row's outputs are zero and the caller redraws f as generatePrivateKeyF does. */
+ * h = (p fq) * g mod (q, x^N-1); rows of N entries, un-trimmed.  Everything runs on the GPU: the inversions modulo 2
+ * and modulo p (the reference's extended Euclid, index.js:425-459) as constant-time divsteps, one warp per key, then
+ * the Newton lifting 2 -> q (index.js:497-509) and h.  Synchronous (host buffers in and out).
+ * valid[b] = 1 iff f_b and g_b are in {-1,0,1} and f_b is invertible modulo 2 and modulo p -- then the outputs equal
+ * the reference's (the inverse is unique); otherwise the row's outputs are zero and the caller redraws f as
+ * generatePrivateKeyF does. */
 int ntru_keygen_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
                       uint8_t *valid);
 
@@ -233,6 +236,20 @@ int ntru_sum_finalize_dev(ntru_ctx *ctx, const uint32_t *partial, uint16_t *out)
  * global row numbers [row0, row0+B) -- index.js:89, 461-488.  The caller owns the row numbering here: never sample
  * two different rows with the same number under one key. */
 int ntru_sample_r_dev(ntru_ctx *ctx, size_t B, int dr, uint64_t row0, uint8_t *r);
+/* ntru_keygen_batch on device rows (pitch ntru_pitch(ctx)), asynchronous on the context's stream; valid: B device bytes.
+ * f, g are int8 (-1 as 0xFF); fq, h uint16; fp bytes in [0,p). */
+int ntru_keygen_dev(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g,
+                    uint16_t *fq, uint8_t *fp, uint16_t *h, uint8_t *valid);
+/* generatePrivateKeyF + generateNewPublicKeyGH for B keys, entirely on the device (index.js:51-79): f drawn with
+ * weights (df, df - 1), g with (dg, dg) (generateCustomArray, index.js:461-488) by the context's ChaCha20 generator;
+ * every f that is not invertible modulo 2 and p is redrawn on the device, for at most 100 rounds in all
+ * (index.js:52-64; then NTRU_E_PARAM "Could not find invertible f").  Every returned row is a valid key pair.
+ * The context owns the row numbers: with R = ntru_rng_next_row at entry, f of key b comes from row R + b and g from
+ * R + B + b; redraw round k >= 1 takes f of key b from row R + (k+1) B + b, and on return the next row is
+ * R + (last round + 2) B.  Each round ends with a 4-byte copy to the host and a stream synchronisation (the count of
+ * rows still to redraw); the lifting and h run once after the last round, asynchronously. */
+int ntru_generate_keys_dev(ntru_ctx *ctx, size_t B, int df, int dg,
+                           int8_t *f, int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h);
 
 /* ---- cross-GPU homomorphic sum (one context = one rank = one GPU of the same node) ----
  * The only exchange step of the hot path: every rank reduces its rows to N column sums mod q and all ranks need the

@@ -19,7 +19,7 @@ NTRU_E_NCCL, NTRU_E_NOMEM, NTRU_E_UNSUPPORTED = -5, -6, -7
 NTRU_OPT_PATH, NTRU_OPT_CHUNK_ROWS, NTRU_OPT_TIMING, NTRU_OPT_DR, NTRU_OPT_DEC1_FORM, NTRU_OPT_SCHEDULE, NTRU_OPT_EPILOGUE = 1, 2, 3, 5, 6, 7, 8
 NTRU_OPT_IMMA_FORM = 9
 KERNEL_KINDS = ["enc_tensor", "dec1_tensor", "dec2_tensor", "enc_core", "dec_core", "sum", "other", "enc_imma", "dec_imma",
-                "muldiv", "pack"]
+                "muldiv", "pack", "inverse"]
 PATH_AUTO, PATH_CUDA_CORE, PATH_TENSOR, PATH_IMMA = 0, 1, 2, 3
 
 #: every symbol include/ntru_b200.h declares: name -> (restype, argtypes)
@@ -53,6 +53,8 @@ SYMBOLS = {
     "ntru_unpack_input": (c_int, [_P, c_size_t, _P, c_int, ctypes.c_uint32, c_int, _P, c_int]),
     "ntru_get_params": (c_int, [_P, POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "ntru_keygen_batch": (c_int, [_P, c_size_t, _P, _P, _P, _P, _P, _P]),
+    "ntru_keygen_dev": (c_int, [_P, c_size_t, _P, _P, _P, _P, _P, _P]),
+    "ntru_generate_keys_dev": (c_int, [_P, c_size_t, c_int, c_int, _P, _P, _P, _P, _P]),
     "ntru_pack_geometry": (c_int, [ctypes.c_uint32, c_int, POINTER(c_int), POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "ntru_pack_output_dev": (c_int, [_P, c_size_t, _P, c_int, c_int, c_size_t, ctypes.c_uint32, _P]),
     "ntru_unpack_input_dev": (c_int, [_P, c_size_t, _P, c_int, ctypes.c_uint32, c_int, _P, c_int, c_size_t]),

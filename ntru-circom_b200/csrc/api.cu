@@ -341,6 +341,7 @@ void ntru_destroy(ntru_ctx *ctx) {
   xchg_release(ctx);
   ctx->d_h.release(); ctx->d_f.release(); ctx->d_fp.release(); ctx->d_b.release(); ctx->d_partial.release(); ctx->d_sum_scratch.release();
   ctx->km_h.mat.release(); ctx->km_f.mat.release(); ctx->km_fp.mat.release();
+  for (auto &b : ctx->kg_bufs) b.release();
   for (auto &t : ctx->timed) {
     cudaEventDestroy(t.a);
     cudaEventDestroy(t.b);
@@ -512,7 +513,7 @@ static int encrypt_host(ntru_ctx *ctx, size_t B, const uint16_t *h, const uint8_
   if (!r) ctx->rng_row += B;                             // a row number (nonce) is never used twice under one key
   return run_pipeline(ctx, B, arr, [&](size_t rows, void **dev) {
     if (!r) {
-      int rs = launch_sample_r(ctx, rows, ctx->opt_dr, next_row, (uint8_t *)dev[1]);
+      int rs = launch_sample(ctx, rows, ctx->opt_dr, ctx->opt_dr, 2, next_row, nullptr, (uint8_t *)dev[1]);
       if (rs) return rs;
       next_row += rows;
     }
@@ -654,6 +655,26 @@ int ntru_keygen_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g,
   if (rc) return rc;
   if (B > 0 && (!f || !g || !fq || !fp || !h || !valid)) return fail(ctx, NTRU_E_PARAM, "f, g, fq, fp, h and valid are required");
   return keygen_batch(ctx, B, f, g, fq, fp, h, valid);
+}
+
+int ntru_keygen_dev(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
+                    uint8_t *valid) {
+  int rc = check(ctx);
+  if (rc) return rc;
+  if (B > 0 && (!f || !g || !fq || !fp || !h || !valid)) return fail(ctx, NTRU_E_PARAM, "f, g, fq, fp, h and valid are required");
+  return keygen_dev(ctx, B, f, g, fq, fp, h, valid);
+}
+
+int ntru_generate_keys_dev(ntru_ctx *ctx, size_t B, int df, int dg, int8_t *f, int8_t *g, uint16_t *fq, uint8_t *fp,
+                           uint16_t *h) {
+  int rc = check(ctx);
+  if (rc) return rc;
+  if (B > 0 && (!f || !g || !fq || !fp || !h)) return fail(ctx, NTRU_E_PARAM, "f, g, fq, fp and h are required");
+  // index.js:462-464 (f has df ones and df - 1 minus ones, g dg of each)
+  if (df < 1 || 2 * df - 1 > ctx->N || dg < 0 || 2 * dg > ctx->N)
+    return fail(ctx, NTRU_E_PARAM, "The total of 1s and -1s cannot exceed the array length.");
+  if (!ctx->rng_keyed) return fail(ctx, NTRU_E_UNSUPPORTED, "the device generator has no key (no OS entropy; call ntru_set_rng_key)");
+  return generate_keys_dev(ctx, B, df, dg, f, g, fq, fp, h);
 }
 
 
@@ -911,7 +932,7 @@ int ntru_sample_r_dev(ntru_ctx *ctx, size_t B, int dr, uint64_t row0, uint8_t *r
   // index.js:462-464
   if (dr < 0 || 2 * dr > ctx->N) return fail(ctx, NTRU_E_PARAM, "The total of 1s and -1s cannot exceed the array length.");
   if (!ctx->rng_keyed) return fail(ctx, NTRU_E_UNSUPPORTED, "the device generator has no key (no OS entropy; call ntru_set_rng_key)");
-  return launch_sample_r(ctx, B, dr, row0, r);
+  return launch_sample(ctx, B, dr, dr, 2, row0, nullptr, r);
 }
 
 int ntru_set_rng_key(ntru_ctx *ctx, const uint8_t key[NTRU_RNG_KEY_BYTES], uint64_t first_row) {

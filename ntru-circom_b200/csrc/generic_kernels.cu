@@ -516,10 +516,11 @@ __global__ void k_sum_finalize(const uint32_t *__restrict__ partial, int N, int 
   if (k < P) out[k] = k < N ? (uint16_t)(partial[k] & qmask) : (uint16_t)0;
 }
 
-// ---- device sampler for r: generateCustomArray(N, dr, dr).map(-1 -> 2) -------------------------
-// Same algorithm as index.js:461-488 (dr ones, dr "minus ones", Fisher-Yates from the top with
-// j = rand32 % (i+1)); the WebCrypto draw (index.js:481-483) is replaced by a keyed counter-mode CSPRNG so that the
-// device can draw r itself (ntru_encrypt_batch with r == NULL) and any row can be replayed by the key holder:
+// ---- device sampler: generateCustomArray(N, ones, neg_ones) ----------------------------------
+// Same algorithm as index.js:461-488 (`ones` ones, `neg_ones` "minus ones", Fisher-Yates from the top with
+// j = rand32 % (i+1)); a -1 is stored as the byte neg_code: 2 for r (generateCustomArray(N, dr, dr).map(-1 -> 2),
+// index.js:89), 0xFF (int8 -1) for the key polynomials f and g (index.js:52-70).  The WebCrypto draw (index.js:481-483)
+// is replaced by a keyed counter-mode CSPRNG so that the device can draw r itself (ntru_encrypt_batch with r == NULL) and any row can be replayed by the key holder:
 // ChaCha20 (D. J. Bernstein's layout: 256-bit key, 64-bit block counter, 64-bit nonce), nonce = global row number,
 // block counter = 0, 1, ... within the row; the draw for position i = N-1, N-2, ..., 1 is keystream word
 // w = N-1-i (word w % 16 of block w / 16).  The key comes from the operating system's entropy (ntru_create) or
@@ -559,15 +560,17 @@ __device__ __forceinline__ void chacha20_block(const ChaChaKey &key, uint64_t co
 
 constexpr int kSampleRows = 64;   // rows (threads) per CTA
 
-__global__ void __launch_bounds__(kSampleRows) k_sample_r(int N, int P, int dr, const ChaChaKey key, uint64_t row0,
-                                                          size_t B, uint8_t *__restrict__ r) {
+// skip (may be NULL): rows b with skip[b] != 0 are neither drawn nor written
+__global__ void __launch_bounds__(kSampleRows) k_sample_ternary(int N, int P, int ones, int neg_ones, uint8_t neg_code,
+                                                                const ChaChaKey key, uint64_t row0, size_t B,
+                                                                const uint8_t *__restrict__ skip, uint8_t *__restrict__ r) {
   extern __shared__ __align__(16) uint8_t arr[];
   const int stride = P + 4;                       // bytes; (P+4)/4 is odd, so rows start in distinct banks
   const size_t first = (size_t)blockIdx.x * kSampleRows;
   const size_t row = first + threadIdx.x;
   uint8_t *mine = arr + (size_t)threadIdx.x * stride;
-  if (row < B) {
-    for (int i = 0; i < P; ++i) mine[i] = i < dr ? 1 : (i < 2 * dr ? 2 : 0);
+  if (row < B && !(skip && skip[row])) {
+    for (int i = 0; i < P; ++i) mine[i] = i < ones ? 1 : (i < ones + neg_ones ? neg_code : 0);
     int i = N - 1;
     for (uint64_t blk = 0; i > 0; ++blk) {
       uint32_t ks[16];
@@ -591,6 +594,7 @@ __global__ void __launch_bounds__(kSampleRows) k_sample_r(int N, int P, int dr, 
   for (size_t idx = threadIdx.x; idx < rows_here * wpr; idx += blockDim.x) {
     const size_t rr = idx / wpr;
     const int w = (int)(idx % wpr);
+    if (skip && skip[first + rr]) continue;
     reinterpret_cast<uint32_t *>(r + (first + rr) * (size_t)P)[w] =
         *reinterpret_cast<const uint32_t *>(arr + rr * stride + 4 * w);
   }
@@ -895,11 +899,12 @@ int launch_sum_finalize(ntru_ctx *ctx, const uint32_t *partial, uint16_t *out) {
   return NTRU_OK;
 }
 
-int launch_sample_r(ntru_ctx *ctx, size_t B, int dr, uint64_t row0, uint8_t *r) {
+int launch_sample(ntru_ctx *ctx, size_t B, int ones, int neg_ones, uint8_t neg_code, uint64_t row0, const uint8_t *skip,
+                  uint8_t *r) {
   if (B == 0) return NTRU_OK;
   const size_t smem = (size_t)kSampleRows * (ctx->P + 4);
   if (!ctx->sampler_attr_set) {
-    NTRU_CUDA(ctx, cudaFuncSetAttribute(k_sample_r, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+    NTRU_CUDA(ctx, cudaFuncSetAttribute(k_sample_ternary, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
     ctx->sampler_attr_set = true;
   }
   ChaChaKey key;
@@ -907,7 +912,8 @@ int launch_sample_r(ntru_ctx *ctx, size_t B, int dr, uint64_t row0, uint8_t *r) 
   const size_t blocks = (B + kSampleRows - 1) / kSampleRows;
   {
     LaunchTimer timer(ctx, NTRU_K_OTHER);
-    k_sample_r<<<(unsigned)blocks, kSampleRows, smem, ctx->stream>>>(ctx->N, ctx->P, dr, key, row0, B, r);
+    k_sample_ternary<<<(unsigned)blocks, kSampleRows, smem, ctx->stream>>>(ctx->N, ctx->P, ones, neg_ones, neg_code, key, row0,
+                                                                            B, skip, r);
   }
   NTRU_CUDA(ctx, cudaGetLastError());
   return NTRU_OK;

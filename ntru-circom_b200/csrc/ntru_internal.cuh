@@ -63,6 +63,7 @@ struct ntru_ctx {
   ntru::DevBuf slot_bufs[ntru::kNumSlots][10];     // pitched device arrays of the host pipeline
   ntru::DevBuf slot_packed[ntru::kNumSlots][10];   // packed staging (what the 1-D H2D / D2H copies move)
   ntru::DevBuf d_partial;
+  ntru::DevBuf kg_bufs[12];         // key generation: lifting scratch (t, u0, u1, r0, r1), host-form rows, valid, count
   ntru::DevBuf d_sum_scratch;      // tree scratch of the ciphertext sum (per-CTA rows, per-group rows, tickets)
   // cross-GPU sum: exchange window (this rank's, cudaMalloc + IPC) and the mapped windows of the peers
   static constexpr int kMaxRanks = 16;
@@ -144,7 +145,10 @@ int launch_sum_finalize(ntru_ctx *ctx, const uint32_t *partial, uint16_t *out);
 size_t xchg_window_bytes(const ntru_ctx *ctx, int world);
 int launch_sum_allreduce(ntru_ctx *ctx, size_t B, const uint16_t *e, uint16_t *out);
 int launch_xchg_partial(ntru_ctx *ctx, uint32_t *partial, uint16_t *out);   // exchange of already accumulated column sums
-int launch_sample_r(ntru_ctx *ctx, size_t B, int dr, uint64_t row0, uint8_t *r);
+// generateCustomArray(N, ones, neg_ones) with -1 stored as neg_code, rows [row0, row0 + B) of the ChaCha20 generator;
+// rows with skip[b] != 0 (skip may be NULL) are left untouched
+int launch_sample(ntru_ctx *ctx, size_t B, int ones, int neg_ones, uint8_t neg_code, uint64_t row0, const uint8_t *skip,
+                  uint8_t *r);
 int launch_wire_unpack(ntru_ctx *ctx, size_t B, const uint32_t *data, int in_elems, int bits, int n, int width, void *out,
                        int elem_bytes);
 int launch_pack_fields(ntru_ctx *ctx, size_t B, const void *data, int elem_bytes, int data_len, size_t pitch, int bits, int n,
@@ -162,9 +166,14 @@ int launch_decrypt_imma(ntru_ctx *ctx, size_t B, const int8_t *f, const uint8_t 
 
 int launch_muldiv_imma(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int mod_p, void *quo, void *rem);
 
-// ---- batched key generation (keygen.cu): host extended Euclid + GPU lifting ----
+// ---- batched key generation (keygen.cu): divstep inversions modulo 2 and 3, IMMA lifting to q and h ----
+constexpr int kKeygenRounds = 100;   // draws of f per key before giving up (index.js:52-64)
+int keygen_dev(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
+               uint8_t *valid);
 int keygen_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
                  uint8_t *valid);
+int generate_keys_dev(ntru_ctx *ctx, size_t B, int df, int dg, int8_t *f, int8_t *g, uint16_t *fq, uint8_t *fp,
+                      uint16_t *h);
 
 // ---- tcgen05 schedule (umma_kernels.cu) ----
 int umma_init(ntru_ctx *ctx);                    // probes the device, sets ctx->tensor_ok

@@ -272,6 +272,20 @@ class Engine:
         self._check(self.lib.ntru_keygen_batch(self._h, B, _ptr(f), _ptr(g), _ptr(fq), _ptr(fp), _ptr(h), _ptr(valid)))
         return {"fq": fq, "fp": fp, "h": h, "valid": valid.astype(bool)}
 
+    def keygen_dev(self, B, f, g, fq, fp, h, valid):
+        """keygen_batch on device rows (pitch self.pitch; f, g int8, fq, h uint16, fp and valid bytes), asynchronous on
+        the context's stream."""
+        self._check(self.lib.ntru_keygen_dev(self._h, B, _ptr(f), _ptr(g), _ptr(fq), _ptr(fp), _ptr(h), _ptr(valid)))
+
+    def generate_keys_dev(self, B, df, dg, f, g, fq, fp, h, seed=None):
+        """generatePrivateKeyF + generateNewPublicKeyGH (index.js:51-79) for B keys into device rows: f, g drawn by the
+        context's ChaCha20 generator (weights (df, df - 1) and (dg, dg)), non-invertible f redrawn on the device.
+        seed: as in sample_r_dev (tests / benchmarks only)."""
+        if seed is not None:
+            self.set_rng_key(seed_key(seed), self.rng_next_row)
+        self._check(self.lib.ntru_generate_keys_dev(self._h, B, int(df), int(dg), _ptr(f), _ptr(g), _ptr(fq), _ptr(fp),
+                                                    _ptr(h)))
+
     def muldiv_dev(self, B, x, y, mod_p, quotient=None, remainder=None):
         """multiplyPolynomials(x, y, mod) + dividePolynomials(., 1 - x^N, mod), device-resident rows."""
         self._check(self.lib.ntru_muldiv_dev(self._h, B, _ptr(x), _ptr(y), int(bool(mod_p)), _ptr(quotient), _ptr(remainder)))
@@ -390,7 +404,7 @@ class Engine:
         self._check(self.lib.ntru_xchg_destroy(self._h))
 
 
-# ---- host copy of the device generator (csrc/generic_kernels.cu: chacha20_block, k_sample_r) -------------------------
+# ---- host copy of the device generator (csrc/generic_kernels.cu: chacha20_block, k_sample_ternary) ------------------
 # For the key holder's audit replay of device-drawn r and for the parity tests; never used to produce r in the product.
 _M32 = 0xFFFFFFFF
 
@@ -426,7 +440,7 @@ def chacha20_block(key: bytes, counter: int, nonce: int):
 
 def sampler_draws(key: bytes, row: int, count: int):
     """The first `count` 32-bit draws of global row number `row`: what the device feeds, in order, to the Fisher-Yates
-    steps i = N-1, N-2, ... of generateCustomArray (index.js:476-485)."""
+    steps i = N-1, N-2, ... of generateCustomArray (index.js:476-485), for r as for the key polynomials f and g."""
     out = []
     blk = 0
     while len(out) < count:

@@ -4,8 +4,9 @@ Same constructor options and defaults, same field and method names, same
 ``{value, inputs, params}`` results (``inputs`` is the key the reference's code
 uses; ``input`` is offered as an alias because the README spells it that way).
 ``encryptBits`` / ``decryptBits`` / ``encryptStr`` / ``decryptStr`` run on the
-GPU through libntru_b200.so; key generation and inversion stay on the host
-(``poly.py``).  Additional batch methods (``encryptBitsBatch``,
+GPU through libntru_b200.so; single-key generation and inversion stay on the host
+(``poly.py``), batched key generation (``generateKeysBatch``, ``generateKeysDevice``)
+runs on the GPU.  Additional batch methods (``encryptBitsBatch``,
 ``decryptBitsBatch``, ``sumCiphertexts``) expose the engine's real unit of
 work: many ciphertexts per call.
 """
@@ -107,8 +108,8 @@ class NTRU:
     def generateKeysBatch(self, B: int) -> dict:
         """B key pairs at once (SURVEY 8f-3): generatePrivateKeyF + generateNewPublicKeyGH (index.js:51-79) with the
         same draws (generateCustomArray with weights (df, df - 1) for f and (dg, dg) for g) and the same retry rule
-        (redraw f while it is not invertible, at most 100 times).  The inversions modulo 2 and p run on the host inside
-        the library, the lifting to q and h on the GPU (ntru_keygen_batch).  Returns fixed-length numpy arrays."""
+        (redraw f while it is not invertible, at most 100 times).  The draws come from rand32 on the host; the inversions,
+        the lifting to q and h run on the GPU (ntru_keygen_batch).  Returns fixed-length numpy arrays."""
         N = self.N
         eng = self.engine()
         f = np.zeros((B, N), dtype=np.int8)
@@ -127,6 +128,22 @@ class NTRU:
         if todo.size:
             raise ValueError("Could not find invertible f")              # index.js:63
         return {"f": f, "g": g, **out}
+
+    def generateKeysDevice(self, B: int) -> dict:
+        """B key pairs drawn and computed entirely on the GPU (ntru_generate_keys_dev): f with weights (df, df - 1), g
+        with (dg, dg) from the engine's ChaCha20 generator, non-invertible f redrawn there (at most 100 rounds).  Returns
+        torch CUDA tensors (B, pitch) f, g (int8), fq, h (int16 holding uint16), fp (uint8), ready to pass as h_rows /
+        f_rows / fp_rows to Engine.encrypt_dev / decrypt_dev.  The tensors are complete on return."""
+        import torch
+        eng = self.engine()
+        dev = torch.device("cuda", eng.device)
+        P = eng.pitch
+        out = {"f": torch.empty((B, P), dtype=torch.int8, device=dev), "g": torch.empty((B, P), dtype=torch.int8, device=dev),
+               "fq": torch.empty((B, P), dtype=torch.int16, device=dev), "fp": torch.empty((B, P), dtype=torch.uint8, device=dev),
+               "h": torch.empty((B, P), dtype=torch.int16, device=dev)}
+        eng.generate_keys_dev(B, self.df, self.dg, out["f"], out["g"], out["fq"], out["fp"], out["h"])
+        eng.sync()
+        return out
 
     def generateNewPublicKeyGH(self):
         self.g = poly.generateCustomArray(self.N, self.dg, self.dg, self.rand32)
