@@ -27,6 +27,11 @@
  *     ntru_last_error(ctx) gives the message.  There is no CPU fallback: without
  *     a CUDA device every compute entry point fails with NTRU_E_CUDA.
  *   - A context is single-caller (one host thread at a time), one per GPU.
+ *   - Ordering.  A context runs on one stream at a time: its own non-blocking stream from ntru_create, or
+ *     the caller's after ntru_set_stream.  Key and option setters apply to the calls made after them;
+ *     calls already queued keep the key and options they were queued with.  ntru_set_stream orders the
+ *     new stream after the work queued on the old one.  Ordering the caller's own input and output
+ *     buffers against ntru_stream(ctx) stays the caller's job.
  */
 #ifndef NTRU_B200_H
 #define NTRU_B200_H
@@ -115,7 +120,9 @@ int ntru_last_path(const ntru_ctx *ctx);
 int ntru_timing_read(ntru_ctx *ctx, int kind, double *total_ms, uint64_t *launches);
 int ntru_timing_reset(ntru_ctx *ctx);
 
-/* this.h = ... (index.js:72-79 result, expanded to N entries in [0,q)) */
+/* this.h = ... (index.js:72-79 result, expanded to N entries in [0,q)).  The key is copied on the context's stream,
+ * after the calls queued there, and the stream is synchronised before the function returns (queued calls finish under
+ * the key they were queued with; the same holds for ntru_set_private_key). */
 int ntru_set_public_key(ntru_ctx *ctx, const uint16_t *h);
 /* this.f, this.fp (index.js:30-36): f in {-1,0,1}, fp expanded to N entries in [0,p) */
 int ntru_set_private_key(ntru_ctx *ctx, const int8_t *f, const uint8_t *fp);
@@ -275,6 +282,9 @@ int ntru_sum_allreduce_dev(ntru_ctx *ctx, size_t B, const uint16_t *e, uint16_t 
 int ntru_xchg_destroy(ntru_ctx *ctx);
 
 void *ntru_stream(ntru_ctx *ctx);              /* cudaStream_t */
+/* The context runs its calls on `stream` from now on (0 = the legacy default stream).  The context's own stream is
+ * synchronised and destroyed; a previous caller stream is not waited for on the host, but the new stream waits for
+ * the work queued on it (that work may still use the context's scratch). */
 int ntru_set_stream(ntru_ctx *ctx, void *stream);
 int ntru_sync(ntru_ctx *ctx);
 

@@ -443,7 +443,10 @@ int ntru_set_public_key(ntru_ctx *ctx, const uint16_t *h) {
     if (h[i] >= ctx->q) return fail(ctx, NTRU_E_PARAM, "h coefficient outside [0,q)");
     tmp[i] = h[i];
   }
-  NTRU_CUDA(ctx, cudaMemcpy(ctx->d_h.ptr, tmp, (size_t)ctx->P * 2, cudaMemcpyHostToDevice));
+  // on the context's stream, so that calls queued before this one finish under the key they were queued with; a plain
+  // cudaMemcpy runs on the legacy stream, which does not wait for a non-blocking one.  tmp lives on this frame.
+  NTRU_CUDA(ctx, cudaMemcpyAsync(ctx->d_h.ptr, tmp, (size_t)ctx->P * 2, cudaMemcpyHostToDevice, ctx->stream));
+  NTRU_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->has_pub = true;
   ctx->km_h.ready = false;
   if (ctx->tensor_ok) {
@@ -467,8 +470,10 @@ int ntru_set_private_key(ntru_ctx *ctx, const int8_t *f, const uint8_t *fp) {
     tf[i] = f[i];
     tp[i] = fp[i];
   }
-  NTRU_CUDA(ctx, cudaMemcpy(ctx->d_f.ptr, tf, (size_t)ctx->P, cudaMemcpyHostToDevice));
-  NTRU_CUDA(ctx, cudaMemcpy(ctx->d_fp.ptr, tp, (size_t)ctx->P, cudaMemcpyHostToDevice));
+  // ordered after the queued calls, as in ntru_set_public_key
+  NTRU_CUDA(ctx, cudaMemcpyAsync(ctx->d_f.ptr, tf, (size_t)ctx->P, cudaMemcpyHostToDevice, ctx->stream));
+  NTRU_CUDA(ctx, cudaMemcpyAsync(ctx->d_fp.ptr, tp, (size_t)ctx->P, cudaMemcpyHostToDevice, ctx->stream));
+  NTRU_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->has_priv = true;
   ctx->km_f.ready = ctx->km_fp.ready = false;
   if (ctx->tensor_ok) {
@@ -950,12 +955,23 @@ uint64_t ntru_rng_next_row(const ntru_ctx *ctx) { return ctx ? ctx->rng_row : 0;
 void *ntru_stream(ntru_ctx *ctx) { return ctx ? (void *)ctx->stream : nullptr; }
 
 int ntru_set_stream(ntru_ctx *ctx, void *stream) {
-  if (!ctx) return NTRU_E_PARAM;
+  int rc = check(ctx);
+  if (rc) return rc;
+  cudaStream_t next = (cudaStream_t)stream;
   if (ctx->own_stream && ctx->stream) {
     cudaStreamSynchronize(ctx->stream);
     cudaStreamDestroy(ctx->stream);
+  } else if (ctx->stream != next) {
+    // calls queued on the caller's old stream may still use scratch the context owns (the lifted b, the sum tree's rows
+    // and tickets, the key-generation buffers, the key matrices): the new stream waits for them
+    cudaEvent_t ev = pool_get(ctx);
+    if (!ev) return fail(ctx, NTRU_E_CUDA, "CUDA error: cudaEventCreate failed in ntru_set_stream");
+    cudaError_t e = cudaEventRecord(ev, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(next, ev, 0);
+    ctx->event_pool.push_back(ev);     // the wait holds on to the recorded work; the event can be recorded again
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "ordering the new stream after the old one (ntru_set_stream)");
   }
-  ctx->stream = (cudaStream_t)stream;
+  ctx->stream = next;
   ctx->own_stream = false;
   return NTRU_OK;
 }
