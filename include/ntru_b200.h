@@ -235,7 +235,8 @@ int ntru_encrypt_dev(ntru_ctx *ctx, size_t B, const uint16_t *h_rows, const uint
 int ntru_decrypt_dev(ntru_ctx *ctx, size_t B, const int8_t *f_rows, const uint8_t *fp_rows, const uint16_t *e,
                      uint8_t *value, uint16_t *quotient1, uint16_t *remainder1,
                      uint8_t *quotient2, uint8_t *remainder2);
-/* partial[k] += sum_b e[b][k] over this call's rows (uint32 wrap-around is exact mod q); partial has pitch entries */
+/* adds the column sums of this call's rows into partial (pitch entries): afterwards each partial[k] is congruent to its
+ * old value plus sum_b e[b][k] modulo 2^16, so modulo q.  It is not the uint32 sum: only its value modulo q is defined. */
 int ntru_sum_partial_dev(ntru_ctx *ctx, size_t B, const uint16_t *e, uint32_t *partial);
 /* out[k] = partial[k] mod q for k < N (and 0 up to pitch) */
 int ntru_sum_finalize_dev(ntru_ctx *ctx, const uint32_t *partial, uint16_t *out);
