@@ -128,6 +128,29 @@ export function accelerate(NTRUReference, ref) {
       }
       return { f, g, ...native.keygenBatch(this.#engine(), B, f, g) };
     }
+    // witness checks (VerifyEncrypt / VerifyDecrypt / VerifyInverse) for B witnesses: inputs under the reference's key
+    // names as flat typed arrays of B rows (h, f, fp may be one row of N), params as the reference emits them.
+    // Returns Uint8Array(B) verdicts: bit 1 satisfied, 2 canonical (what dividePolynomials returns), 4 not evaluated.
+    #checkParams(params, want, what) {
+      if (params.length !== want.length || params.some((x, i) => Number(x) !== want[i]))
+        throw new Error(`${what} params ${params} do not match this instance's ${want}`);
+    }
+    verifyEncryptBatch(B, inputs, params) {
+      this.#checkParams(params, [this.q, this.calculateNq(), this.N], 'VerifyEncrypt');
+      const { h, r, m, quotientE, remainderE } = inputs;
+      return native.checkEncryptBatch(this.#engine(), B, h, h.length === this.N, r, m, quotientE, remainderE);
+    }
+    verifyDecryptBatch(B, inputs, params) {
+      this.#checkParams(params, [this.q, this.calculateNq(), this.p, this.calculateNp(), this.N], 'VerifyDecrypt');
+      const { f, fp, e, quotient1, remainder1, quotient2, remainder2 } = inputs;
+      return native.checkDecryptBatch(this.#engine(), B, f, fp, f.length === this.N, e, quotient1, remainder1, quotient2, remainder2);
+    }
+    verifyInverseBatch(B, inputs, params) {
+      const modP = Number(params[0]) === this.p;
+      this.#checkParams(params, modP ? [this.p, this.calculateNp(), this.N] : [this.q, this.calculateNq(), this.N], 'VerifyInverse');
+      const { f, fq, quotientI, remainderI } = inputs;
+      return native.checkInverseBatch(this.#engine(), B, modP, f, fq, quotientI, remainderI);
+    }
     close() { if (this.#ctx) { native.destroy(this.#ctx); this.#ctx = null; this.#pub = this.#priv = null; } }
   };
 }

@@ -22,6 +22,11 @@
  *   encryptBatchPacked(handle, B, r: Uint32Array | null, m: Uint32Array) / decryptBatchPacked(handle, B, e: Uint32Array):
  *        the same with every array as rows of BN254 field elements (packOutput form), B x packedElems x 8 words
  *   verifyKeysBatch(handle, B, f, fq, fp, g)   keygenBatch(handle, B, f, g)
+ *   checkEncryptBatch(handle, B, h, keyShared, r, m, quotientE, remainderE) -> Uint8Array(B) verdicts
+ *   checkDecryptBatch(handle, B, f, fp, keyShared, e, quotient1, remainder1, quotient2, remainder2) -> Uint8Array(B)
+ *   checkInverseBatch(handle, B, modP, x, y, quotientI, remainderI) -> Uint8Array(B)
+ *        witness checks (VerifyEncrypt / VerifyDecrypt / VerifyInverse): bit 1 satisfied, 2 canonical, 4 not evaluated;
+ *        keyShared: h (f, fp) is one row of N; y, quotientI, remainderI are Uint8Array when modP
  *   packOutput(handle, B, maxVal, data: Uint8Array | Uint16Array, dataLen) -> Uint32Array(B x outputSize x 8)
  *   unpackInput(handle, B, maxVal, packedBits, data: Uint32Array, nElems, wide: bool) -> Uint8Array | Uint16Array
  *   packGeometry(maxVal, dataLen) -> {maxInputBits, inputsPerOutput, arrLen, outputSize}
@@ -448,6 +453,93 @@ static napi_value KeygenBatch(napi_env env, napi_callback_info info) {
   return out;
 }
 
+/* ---- witness checks: VerifyEncrypt / VerifyDecrypt / VerifyInverse (circuits/ntru.circom:155-256) ----------------- */
+static bool get_flag(napi_env env, napi_value v, bool *out) {
+  *out = false;
+  return is_nullish(env, v) || napi_get_value_bool(env, v, out) == napi_ok;
+}
+
+static napi_value CheckEncryptBatch(napi_env env, napi_callback_info info) {
+  ARGS(8);
+  ntru_ctx *ctx = get_ctx(env, argv[0]);
+  size_t N;
+  uint32_t B;
+  bool shared;
+  if (!ctx || !ctx_N(ctx, &N) || !get_u32(env, argv[1], &B, "B: row count")) return NULL;
+  if (!get_flag(env, argv[3], &shared)) { napi_throw_type_error(env, NULL, "keyShared: boolean"); return NULL; }
+  const size_t rows = (size_t)B * N, wit = (size_t)B * (N + 1);
+  const uint16_t *h = (const uint16_t *)typed_arg(env, argv[2], napi_uint16_array, shared ? N : rows, "h: Uint16Array(N or B x N)");
+  if (!h) return NULL;
+  const uint8_t *r = (const uint8_t *)typed_arg(env, argv[4], napi_uint8_array, rows, "r: Uint8Array(B x N)");
+  if (!r) return NULL;
+  const uint16_t *m = (const uint16_t *)typed_arg(env, argv[5], napi_uint16_array, rows, "m: Uint16Array(B x N)");
+  if (!m) return NULL;
+  const uint16_t *qe = (const uint16_t *)typed_arg(env, argv[6], napi_uint16_array, wit, "quotientE: Uint16Array(B x (N+1))");
+  if (!qe) return NULL;
+  const uint16_t *re = (const uint16_t *)typed_arg(env, argv[7], napi_uint16_array, wit, "remainderE: Uint16Array(B x (N+1))");
+  if (!re) return NULL;
+  void *verdict;
+  napi_value out = make_typed(env, napi_uint8_array, B, 1, &verdict);
+  if (!verdict) return NULL;
+  NTRU_TRY(env, ctx, ntru_check_encrypt_batch(ctx, B, h, shared, r, m, qe, re, verdict));
+  return out;
+}
+
+static napi_value CheckDecryptBatch(napi_env env, napi_callback_info info) {
+  ARGS(10);
+  ntru_ctx *ctx = get_ctx(env, argv[0]);
+  size_t N;
+  uint32_t B;
+  bool shared;
+  if (!ctx || !ctx_N(ctx, &N) || !get_u32(env, argv[1], &B, "B: row count")) return NULL;
+  if (!get_flag(env, argv[4], &shared)) { napi_throw_type_error(env, NULL, "keyShared: boolean"); return NULL; }
+  const size_t rows = (size_t)B * N, wit = (size_t)B * (N + 1), key = shared ? N : rows;
+  const uint16_t *f = (const uint16_t *)typed_arg(env, argv[2], napi_uint16_array, key, "f: Uint16Array(N or B x N), -1 as q-1");
+  if (!f) return NULL;
+  const uint8_t *fp = (const uint8_t *)typed_arg(env, argv[3], napi_uint8_array, key, "fp: Uint8Array(N or B x N)");
+  if (!fp) return NULL;
+  const uint16_t *e = (const uint16_t *)typed_arg(env, argv[5], napi_uint16_array, rows, "e: Uint16Array(B x N)");
+  if (!e) return NULL;
+  const uint16_t *q1 = (const uint16_t *)typed_arg(env, argv[6], napi_uint16_array, wit, "quotient1: Uint16Array(B x (N+1))");
+  if (!q1) return NULL;
+  const uint16_t *r1 = (const uint16_t *)typed_arg(env, argv[7], napi_uint16_array, wit, "remainder1: Uint16Array(B x (N+1))");
+  if (!r1) return NULL;
+  const uint8_t *q2 = (const uint8_t *)typed_arg(env, argv[8], napi_uint8_array, wit, "quotient2: Uint8Array(B x (N+1))");
+  if (!q2) return NULL;
+  const uint8_t *r2 = (const uint8_t *)typed_arg(env, argv[9], napi_uint8_array, wit, "remainder2: Uint8Array(B x (N+1))");
+  if (!r2) return NULL;
+  void *verdict;
+  napi_value out = make_typed(env, napi_uint8_array, B, 1, &verdict);
+  if (!verdict) return NULL;
+  NTRU_TRY(env, ctx, ntru_check_decrypt_batch(ctx, B, f, fp, shared, e, q1, r1, q2, r2, verdict));
+  return out;
+}
+
+static napi_value CheckInverseBatch(napi_env env, napi_callback_info info) {
+  ARGS(7);
+  ntru_ctx *ctx = get_ctx(env, argv[0]);
+  size_t N;
+  uint32_t B;
+  bool mod_p;
+  if (!ctx || !ctx_N(ctx, &N) || !get_u32(env, argv[1], &B, "B: row count")) return NULL;
+  if (!get_flag(env, argv[2], &mod_p)) { napi_throw_type_error(env, NULL, "modP: boolean"); return NULL; }
+  const size_t rows = (size_t)B * N, wit = (size_t)B * (N + 1);
+  const napi_typedarray_type t = mod_p ? napi_uint8_array : napi_uint16_array;
+  const uint16_t *x = (const uint16_t *)typed_arg(env, argv[3], napi_uint16_array, rows, "x: Uint16Array(B x N)");
+  if (!x) return NULL;
+  const void *y = typed_arg(env, argv[4], t, rows, "y: Uint16Array(B x N), Uint8Array when modP");
+  if (!y) return NULL;
+  const void *qi = typed_arg(env, argv[5], t, wit, "quotientI: Uint16Array(B x (N+1)), Uint8Array when modP");
+  if (!qi) return NULL;
+  const void *ri = typed_arg(env, argv[6], t, wit, "remainderI: Uint16Array(B x (N+1)), Uint8Array when modP");
+  if (!ri) return NULL;
+  void *verdict;
+  napi_value out = make_typed(env, napi_uint8_array, B, 1, &verdict);
+  if (!verdict) return NULL;
+  NTRU_TRY(env, ctx, ntru_check_inverse_batch(ctx, B, mod_p, x, y, qi, ri, verdict));
+  return out;
+}
+
 /* ---- packOutput / unpackInput (index.js:572-620) ----------------------------------------------------------------- */
 static napi_value PackGeometry(napi_env env, napi_callback_info info) {
   ARGS(2);
@@ -586,7 +678,8 @@ static napi_value Init(napi_env env, napi_value exports) {
       FN("decryptBatchPacked", DecryptBatchPacked), FN("verifyKeysBatch", VerifyKeysBatch),
       FN("keygenBatch", KeygenBatch), FN("packGeometry", PackGeometry), FN("packOutput", PackOutput), FN("unpackInput", UnpackInput),
       FN("sum", Sum), FN("xchgCreate", XchgCreate), FN("xchgConnect", XchgConnect), FN("xchgDestroy", XchgDestroy),
-      FN("sumAllreduce", SumAllreduce),
+      FN("sumAllreduce", SumAllreduce), FN("checkEncryptBatch", CheckEncryptBatch), FN("checkDecryptBatch", CheckDecryptBatch),
+      FN("checkInverseBatch", CheckInverseBatch),
   };
 #undef FN
   if (napi_define_properties(env, exports, sizeof d / sizeof d[0], d) != napi_ok) {

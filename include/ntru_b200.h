@@ -97,7 +97,8 @@ enum {
   NTRU_K_MULDIV = 9,        /* mma.sync (IMMA) multiply + divide by 1 - x^N (verifyKeysInputs products) */
   NTRU_K_PACK = 10,         /* packOutput / unpackInput bit packing */
   NTRU_K_INVERSE = 11,      /* key generation: f^-1 modulo 2 and modulo 3 (divsteps) */
-  NTRU_K_COUNT = 12
+  NTRU_K_CHECK = 12,        /* mma.sync (IMMA) witness checks (ntru_check_*) */
+  NTRU_K_COUNT = 13
 };
 
 /* new NTRU({N,p,q}) -- index.js:8-28.  p must be 3, q a power of two in [4, 8192], 8 <= N <= 1024
@@ -185,6 +186,41 @@ int ntru_muldiv_dev(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int
  * generatePrivateKeyF does. */
 int ntru_keygen_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
                       uint8_t *valid);
+
+/* Witness checks -- the constraint systems of VerifyEncrypt, VerifyDecrypt and VerifyInverse
+ * (circuits/ntru.circom:155-256) evaluated for B witnesses at once.  One verdict byte per row:
+ *   NTRU_CHECK_SATISFIED  the constraints hold (for decrypt: both divisions), computed on the raw witness values;
+ *   NTRU_CHECK_CANONICAL  satisfied, every quotient / remainder entry below its modulus and remainder[N] == 0: the arrays
+ *                         are exactly what dividePolynomials returns (expanded to N + 1), i.e. what this library and the
+ *                         reference emit.  The constraints alone accept more: adding t to quotient[0] and remainder[N]
+ *                         and subtracting it from remainder[0], or raising any entry by a multiple of the modulus;
+ *   NTRU_CHECK_DOMAIN     not evaluated (bits 1 and 2 clear): an entry of the small operand (r, f, or the x of
+ *                         VerifyInverse), reduced modulo the product's modulus M, is outside {M-1, 0, 1, 2}.
+ * Witness forms as the reference's `inputs`: r bytes; f, m, e, h, fq, the inverse's x and y uint16 (-1 as q-1 or p-1;
+ * y = fq or the un-reduced p*fq), except y, quotientI and remainderI as bytes when mod_p != 0 (the fp case); quotient2,
+ * remainder2 bytes.  h, e, m are taken modulo q and fp modulo 3 at any value; the lift of decrypt reads the raw
+ * remainder1.  Columns >= N of the inputs and >= N + 1 of the witness arrays are ignored.  Supports N <= 832
+ * (NTRU_E_UNSUPPORTED above).  Every array is required when B > 0 (NTRU_E_PARAM); bad values are not an error, they
+ * are what the verdict reports.
+ * Device form: rows of pitch ntru_pitch(ctx) elements; key_stride = 0 (one key row for every witness) or ntru_pitch(ctx)
+ * (NTRU_E_PARAM otherwise); verdict: B device bytes, exactly B written; asynchronous on the context's stream. */
+enum { NTRU_CHECK_SATISFIED = 1, NTRU_CHECK_CANONICAL = 2, NTRU_CHECK_DOMAIN = 4 };
+int ntru_check_encrypt_dev(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t key_stride, const uint8_t *r,
+                           const uint16_t *m, const uint16_t *quotientE, const uint16_t *remainderE, uint8_t *verdict);
+int ntru_check_decrypt_dev(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, size_t key_stride,
+                           const uint16_t *e, const uint16_t *quotient1, const uint16_t *remainder1,
+                           const uint8_t *quotient2, const uint8_t *remainder2, uint8_t *verdict);
+int ntru_check_inverse_dev(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y,
+                           const void *quotientI, const void *remainderI, uint8_t *verdict);
+/* Host form: packed rows (pitch N for the inputs, N + 1 for quotient / remainder), verdict B host bytes; key_shared != 0:
+ * h (or f and fp) is one row of N entries for every witness.  Synchronous. */
+int ntru_check_encrypt_batch(ntru_ctx *ctx, size_t B, const uint16_t *h, int key_shared, const uint8_t *r, const uint16_t *m,
+                             const uint16_t *quotientE, const uint16_t *remainderE, uint8_t *verdict);
+int ntru_check_decrypt_batch(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, int key_shared, const uint16_t *e,
+                             const uint16_t *quotient1, const uint16_t *remainder1, const uint8_t *quotient2,
+                             const uint8_t *remainder2, uint8_t *verdict);
+int ntru_check_inverse_batch(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y,
+                             const void *quotientI, const void *remainderI, uint8_t *verdict);
 
 /* packOutput / unpackInput -- index.js:572-620: coefficients <-> BN254 field elements (CombineArray / UnpackArray,
  * circuits/ntru.circom:259-306).  A field element is 32 bytes, little-endian.

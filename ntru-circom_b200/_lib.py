@@ -19,7 +19,9 @@ NTRU_E_NCCL, NTRU_E_NOMEM, NTRU_E_UNSUPPORTED = -5, -6, -7
 NTRU_OPT_PATH, NTRU_OPT_CHUNK_ROWS, NTRU_OPT_TIMING, NTRU_OPT_DR, NTRU_OPT_DEC1_FORM, NTRU_OPT_SCHEDULE, NTRU_OPT_EPILOGUE = 1, 2, 3, 5, 6, 7, 8
 NTRU_OPT_IMMA_FORM = 9
 KERNEL_KINDS = ["enc_tensor", "dec1_tensor", "dec2_tensor", "enc_core", "dec_core", "sum", "other", "enc_imma", "dec_imma",
-                "muldiv", "pack", "inverse"]
+                "muldiv", "pack", "inverse", "check"]
+#: verdict bits of the witness checks (ntru_check_*)
+NTRU_CHECK_SATISFIED, NTRU_CHECK_CANONICAL, NTRU_CHECK_DOMAIN = 1, 2, 4
 PATH_AUTO, PATH_CUDA_CORE, PATH_TENSOR, PATH_IMMA = 0, 1, 2, 3
 
 #: every symbol include/ntru_b200.h declares: name -> (restype, argtypes)
@@ -60,6 +62,12 @@ SYMBOLS = {
     "ntru_unpack_input_dev": (c_int, [_P, c_size_t, _P, c_int, ctypes.c_uint32, c_int, _P, c_int, c_size_t]),
     "ntru_verify_keys_batch": (c_int, [_P, c_size_t, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "ntru_muldiv_dev": (c_int, [_P, c_size_t, _P, _P, c_int, _P, _P]),
+    "ntru_check_encrypt_dev": (c_int, [_P, c_size_t, _P, c_size_t, _P, _P, _P, _P, _P]),
+    "ntru_check_decrypt_dev": (c_int, [_P, c_size_t, _P, _P, c_size_t, _P, _P, _P, _P, _P, _P]),
+    "ntru_check_inverse_dev": (c_int, [_P, c_size_t, c_int, _P, _P, _P, _P, _P]),
+    "ntru_check_encrypt_batch": (c_int, [_P, c_size_t, _P, c_int, _P, _P, _P, _P, _P]),
+    "ntru_check_decrypt_batch": (c_int, [_P, c_size_t, _P, _P, c_int, _P, _P, _P, _P, _P, _P]),
+    "ntru_check_inverse_batch": (c_int, [_P, c_size_t, c_int, _P, _P, _P, _P, _P]),
     "ntru_encrypt_dev": (c_int, [_P, c_size_t, _P, _P, _P, _P, _P, _P]),
     "ntru_decrypt_dev": (c_int, [_P, c_size_t, _P, _P, _P, _P, _P, _P, _P, _P]),
     "ntru_sum_partial_dev": (c_int, [_P, c_size_t, _P, _P]),

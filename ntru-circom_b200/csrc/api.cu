@@ -63,6 +63,8 @@ struct HostArr {
   // field-element wire format (ntru_*_batch_packed): the host row is fe_elems BN254 field elements of 32 bytes,
   // packOutput(maxVal, width, row).expected -- fe_n coefficients of fe_bits bits each per element; 0 = plain rows
   int fe_bits = 0, fe_n = 0, fe_elems = 0;
+  // flat: one value per row (the verdict bytes of the witness checks): the kernel works on the packed staging itself
+  bool flat = false;
   size_t host_row_bytes() const { return fe_bits ? (size_t)fe_elems * 32 : width * elem; }
 };
 
@@ -78,7 +80,7 @@ int run_pipeline(ntru_ctx *ctx, size_t B, HostArr (&arr)[kMaxArr], Launch launch
   for (int s = 0; s < kNumSlots; ++s)
     for (int a = 0; a < kMaxArr; ++a)
       if (arr[a].used) {
-        NTRU_CUDA(ctx, ctx->slot_bufs[s][a].reserve(rows_alloc * P * arr[a].elem));
+        if (!arr[a].flat) NTRU_CUDA(ctx, ctx->slot_bufs[s][a].reserve(rows_alloc * P * arr[a].elem));
         NTRU_CUDA(ctx, ctx->slot_packed[s][a].reserve(rows_alloc * arr[a].host_row_bytes()));
       }
   size_t ci = 0;
@@ -86,7 +88,8 @@ int run_pipeline(ntru_ctx *ctx, size_t B, HostArr (&arr)[kMaxArr], Launch launch
     const size_t rows = (B - row0) < chunk ? (B - row0) : chunk;
     const int s = (int)(ci % kNumSlots);
     void *dev[kMaxArr];
-    for (int a = 0; a < kMaxArr; ++a) dev[a] = arr[a].used ? ctx->slot_bufs[s][a].ptr : nullptr;
+    for (int a = 0; a < kMaxArr; ++a)
+      dev[a] = arr[a].used ? (arr[a].flat ? ctx->slot_packed[s][a].ptr : ctx->slot_bufs[s][a].ptr) : nullptr;
     // inputs: packed 1-D H2D on s_in (the slot's packed staging is free once the previous unpack ran)
     if (ci >= (size_t)kNumSlots) NTRU_CUDA(ctx, cudaStreamWaitEvent(ctx->s_in, ctx->ev_comp[s], 0));
     for (int a = 0; a < kMaxArr; ++a) {
@@ -109,7 +112,7 @@ int run_pipeline(ntru_ctx *ctx, size_t B, HostArr (&arr)[kMaxArr], Launch launch
     int rc = launch(rows, dev);
     if (rc != NTRU_OK) return rc;
     for (int a = 0; a < kMaxArr; ++a) {
-      if (!arr[a].used || !arr[a].out) continue;
+      if (!arr[a].used || !arr[a].out || arr[a].flat) continue;
       rc = arr[a].fe_bits
                ? launch_pack_fields(ctx, rows, dev[a], (int)arr[a].elem, (int)arr[a].width, (size_t)ctx->P, arr[a].fe_bits, arr[a].fe_n,
                                     arr[a].fe_elems, (uint32_t *)ctx->slot_packed[s][a].ptr)
@@ -342,6 +345,7 @@ void ntru_destroy(ntru_ctx *ctx) {
   ctx->d_h.release(); ctx->d_f.release(); ctx->d_fp.release(); ctx->d_b.release(); ctx->d_partial.release(); ctx->d_sum_scratch.release();
   ctx->km_h.mat.release(); ctx->km_f.mat.release(); ctx->km_fp.mat.release();
   for (auto &b : ctx->kg_bufs) b.release();
+  for (auto &b : ctx->check_key) b.release();
   for (auto &t : ctx->timed) {
     cudaEventDestroy(t.a);
     cudaEventDestroy(t.b);
@@ -680,6 +684,123 @@ int ntru_generate_keys_dev(ntru_ctx *ctx, size_t B, int df, int dg, int8_t *f, i
     return fail(ctx, NTRU_E_PARAM, "The total of 1s and -1s cannot exceed the array length.");
   if (!ctx->rng_keyed) return fail(ctx, NTRU_E_UNSUPPORTED, "the device generator has no key (no OS entropy; call ntru_set_rng_key)");
   return generate_keys_dev(ctx, B, df, dg, f, g, fq, fp, h);
+}
+
+
+// ---- witness checks ------------------------------------------------------------------------------------------------
+
+static int check_args(ntru_ctx *ctx, size_t B, bool all_given, size_t key_stride) {
+  if (!ctx) return NTRU_E_PARAM;
+  if (B > 0 && !all_given) return fail(ctx, NTRU_E_PARAM, "every array of the witness check is required");
+  if (key_stride != 0 && key_stride != (size_t)ctx->P) return fail(ctx, NTRU_E_PARAM, "key_stride must be 0 or ntru_pitch(ctx)");
+  int rc = check(ctx);
+  if (rc) return rc;
+  if (!ctx->tensor_ok) return fail(ctx, NTRU_E_UNSUPPORTED, "witness checks need the sm_100 tensor path");
+  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "witness checks support N <= 832");
+  return NTRU_OK;
+}
+
+int ntru_check_encrypt_dev(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t key_stride, const uint8_t *r, const uint16_t *m,
+                           const uint16_t *quotientE, const uint16_t *remainderE, uint8_t *verdict) {
+  int rc = check_args(ctx, B, h && r && m && quotientE && remainderE && verdict, key_stride);
+  if (rc) return rc;
+  return launch_check_encrypt(ctx, B, h, key_stride, r, m, quotientE, remainderE, verdict);
+}
+
+int ntru_check_decrypt_dev(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, size_t key_stride, const uint16_t *e,
+                           const uint16_t *quotient1, const uint16_t *remainder1, const uint8_t *quotient2,
+                           const uint8_t *remainder2, uint8_t *verdict) {
+  int rc = check_args(ctx, B, f && fp && e && quotient1 && remainder1 && quotient2 && remainder2 && verdict, key_stride);
+  if (rc) return rc;
+  return launch_check_decrypt(ctx, B, f, fp, key_stride, e, quotient1, remainder1, quotient2, remainder2, verdict);
+}
+
+int ntru_check_inverse_dev(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y, const void *quotientI,
+                           const void *remainderI, uint8_t *verdict) {
+  int rc = check_args(ctx, B, x && y && quotientI && remainderI && verdict, 0);
+  if (rc) return rc;
+  return launch_check_inverse(ctx, B, mod_p, x, y, quotientI, remainderI, verdict);
+}
+
+// the shared key row of a host-form check: one upload on the context's stream, ahead of the chunks' kernels
+static int upload_key_row(ntru_ctx *ctx, int slot, const void *row, size_t elem) {
+  const size_t P = (size_t)ctx->P;
+  NTRU_CUDA(ctx, ctx->check_key[slot].reserve(P * elem));
+  NTRU_CUDA(ctx, cudaMemsetAsync(ctx->check_key[slot].ptr, 0, P * elem, ctx->stream));
+  NTRU_CUDA(ctx, cudaMemcpyAsync(ctx->check_key[slot].ptr, row, (size_t)ctx->N * elem, cudaMemcpyHostToDevice, ctx->stream));
+  return NTRU_OK;
+}
+
+int ntru_check_encrypt_batch(ntru_ctx *ctx, size_t B, const uint16_t *h, int key_shared, const uint8_t *r, const uint16_t *m,
+                             const uint16_t *quotientE, const uint16_t *remainderE, uint8_t *verdict) {
+  int rc = check_args(ctx, B, h && r && m && quotientE && remainderE && verdict, 0);
+  if (rc || B == 0) return rc;
+  const size_t N = (size_t)ctx->N;
+  HostArr arr[kMaxArr];
+  if (key_shared) {
+    rc = upload_key_row(ctx, 0, h, 2);
+    if (rc) return rc;
+  } else {
+    set_in(arr[0], h, 2, N);
+  }
+  set_in(arr[1], r, 1, N);
+  set_in(arr[2], m, 2, N);
+  set_in(arr[3], quotientE, 2, N + 1);
+  set_in(arr[4], remainderE, 2, N + 1);
+  set_out(arr[5], verdict, 1, 1);
+  arr[5].flat = true;
+  return run_pipeline(ctx, B, arr, [&](size_t rows, void **dev) {
+    return launch_check_encrypt(ctx, rows, key_shared ? (const uint16_t *)ctx->check_key[0].ptr : (const uint16_t *)dev[0],
+                                key_shared ? 0 : (size_t)ctx->P, (const uint8_t *)dev[1], (const uint16_t *)dev[2],
+                                (const uint16_t *)dev[3], (const uint16_t *)dev[4], (uint8_t *)dev[5]);
+  });
+}
+
+int ntru_check_decrypt_batch(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, int key_shared, const uint16_t *e,
+                             const uint16_t *quotient1, const uint16_t *remainder1, const uint8_t *quotient2,
+                             const uint8_t *remainder2, uint8_t *verdict) {
+  int rc = check_args(ctx, B, f && fp && e && quotient1 && remainder1 && quotient2 && remainder2 && verdict, 0);
+  if (rc || B == 0) return rc;
+  const size_t N = (size_t)ctx->N;
+  HostArr arr[kMaxArr];
+  if (key_shared) {
+    rc = upload_key_row(ctx, 0, f, 2);
+    if (!rc) rc = upload_key_row(ctx, 1, fp, 1);
+    if (rc) return rc;
+  } else {
+    set_in(arr[0], f, 2, N);
+    set_in(arr[1], fp, 1, N);
+  }
+  set_in(arr[2], e, 2, N);
+  set_in(arr[3], quotient1, 2, N + 1);
+  set_in(arr[4], remainder1, 2, N + 1);
+  set_in(arr[5], quotient2, 1, N + 1);
+  set_in(arr[6], remainder2, 1, N + 1);
+  set_out(arr[7], verdict, 1, 1);
+  arr[7].flat = true;
+  return run_pipeline(ctx, B, arr, [&](size_t rows, void **dev) {
+    return launch_check_decrypt(ctx, rows, key_shared ? (const uint16_t *)ctx->check_key[0].ptr : (const uint16_t *)dev[0],
+                                key_shared ? (const uint8_t *)ctx->check_key[1].ptr : (const uint8_t *)dev[1],
+                                key_shared ? 0 : (size_t)ctx->P, (const uint16_t *)dev[2], (const uint16_t *)dev[3],
+                                (const uint16_t *)dev[4], (const uint8_t *)dev[5], (const uint8_t *)dev[6], (uint8_t *)dev[7]);
+  });
+}
+
+int ntru_check_inverse_batch(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y, const void *quotientI,
+                             const void *remainderI, uint8_t *verdict) {
+  int rc = check_args(ctx, B, x && y && quotientI && remainderI && verdict, 0);
+  if (rc || B == 0) return rc;
+  const size_t N = (size_t)ctx->N, wb = mod_p ? 1 : 2;
+  HostArr arr[kMaxArr];
+  set_in(arr[0], x, 2, N);
+  set_in(arr[1], y, wb, N);
+  set_in(arr[2], quotientI, wb, N + 1);
+  set_in(arr[3], remainderI, wb, N + 1);
+  set_out(arr[4], verdict, 1, 1);
+  arr[4].flat = true;
+  return run_pipeline(ctx, B, arr, [&](size_t rows, void **dev) {
+    return launch_check_inverse(ctx, rows, mod_p, (const uint16_t *)dev[0], dev[1], dev[2], dev[3], (uint8_t *)dev[4]);
+  });
 }
 
 

@@ -633,6 +633,322 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_muldiv_imma(const ImmaMulDi
   }
 }
 
+// ---- witness checks: VerifyEncrypt / VerifyDecrypt / VerifyInverse (circuits/ntru.circom:155-256) ------------------
+// One warp per witness row, the product of k_muldiv_imma (x signed in [-1, 2], y any uint16, one accumulator set per
+// limb), and an epilogue that compares instead of storing.  With a = the 2N - 1 coefficients of lin(x, y) (+ m on the
+// first N for encrypt) and Q, R the N + 1 entries of the witness, the division by I = 1 - x^N modulo M holds iff
+//     k < N:  Q[k] + R[k] = a[k]      k = N:  Q[N] - Q[0] + R[N] = a[N]      1 <= k <= N:  Q[k] + a[k + N] = 0
+// (a[k] = 0 for k >= 2N - 1: the last two rows are Q[N-1] = Q[N] = 0).  Every operand is read as the raw witness value,
+// reduced modulo M only where the constraint reduces it.  The witness is canonical -- the arrays dividePolynomials
+// returns -- iff it also has every entry below M and R[N] = 0.
+struct CheckArgs {
+  ImmaLayout L;
+  uint32_t M;               // modulus of the (first) division: q, or p for the mod-p inverse
+  size_t B;
+  const void *x;            // small operand in its witness form: r (bytes), f or x (uint16)
+  const void *y;            // h, e (uint16), or the inverse's y (uint16; bytes modulo p)
+  size_t x_stride, y_stride;   // elements between rows (0: one row for every witness)
+  const uint16_t *m;        // encrypt
+  const uint8_t *fp;        // decrypt (row stride x_stride)
+  const void *quo, *rem;    // the (first) division's witness, uint16 (bytes for the mod-p inverse)
+  const uint8_t *quo2, *rem2;   // decrypt: the second division's witness
+  uint8_t *verdict;
+};
+
+// x operand, witness form -> the signed bytes the product takes: v mod M, with M - 1 as -1.  Columns >= N become 0.
+// Returns false when an entry of this lane lies outside {M - 1, 0, 1, 2} (the row is not evaluated then).
+template <bool U16>
+__device__ __forceinline__ bool stage_small(int N, int P, uint32_t M, const uint8_t *src, uint8_t *xs, int lane) {
+  bool ok = true;
+  for (int j0 = 8 * lane; j0 < P; j0 += 256) {
+    uint32_t w[2] = {0u, 0u};
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const uint32_t v = U16 ? reinterpret_cast<const uint16_t *>(src)[j0 + i] : src[j0 + i];
+      const uint32_t r = M == 3 ? mod3_16(v) : v & (M - 1);
+      const bool valid = j0 + i < N;
+      ok = ok && (!valid || r <= 2u || r == M - 1);
+      const uint32_t s = r == M - 1 ? 0xffu : (r <= 2u ? r : 0u);
+      w[i >> 2] |= (valid ? s : 0u) << (8 * (i & 3));
+    }
+    *reinterpret_cast<uint2 *>(xs + j0) = make_uint2(w[0], w[1]);
+  }
+  return ok;
+}
+
+// bytes -> reversed array, every byte reduced modulo 3 (stage_rev8 copies them as they are)
+__device__ __forceinline__ void stage_rev8_mod3(int N, int Z, const uint8_t *src, uint8_t *y, int lane) {
+  for (int j0 = 16 * lane; j0 < N; j0 += 512) {
+    const uint4 v = *reinterpret_cast<const uint4 *>(src + j0);
+    uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      uint32_t o = 0;
+#pragma unroll
+      for (int b = 0; b < 4; ++b) o |= mod3_16((w[i] >> (8 * b)) & 0xffu) << (8 * b);
+      w[i] = o;
+    }
+    *reinterpret_cast<uint4 *>(y + (Z - j0 - 15)) =
+        make_uint4(__byte_perm(w[3], 0u, 0x0123), __byte_perm(w[2], 0u, 0x0123), __byte_perm(w[1], 0u, 0x0123), __byte_perm(w[0], 0u, 0x0123));
+  }
+}
+
+// packed uint16 lanes of the 8 coefficients k0 .. k0+7 with lo_k <= k <= hi_k
+__device__ __forceinline__ uint32_t lane_mask2(int k0, int i, int lo_k, int hi_k) {
+  const int k = k0 + 2 * i;
+  return (k >= lo_k && k <= hi_k ? 0xffffu : 0u) | (k + 1 >= lo_k && k + 1 <= hi_k ? 0xffff0000u : 0u);
+}
+
+// One pass of a division modulo M = 2^logq (uint16 witness): this lane's coefficients k0 .. k0+7.  lo, hi = product
+// coefficients k and k + N; mv = m (encrypt) or 0; q0 = Q[0].  Mismatches go to bad, canonical-form violations to nonc.
+__device__ __forceinline__ void check_pass_q(int N, int k0, uint32_t Q2, const uint32_t (&lo)[4], const uint32_t (&hi)[4],
+                                             const uint32_t (&mv)[4], const uint32_t (&qv)[4], const uint32_t (&rv)[4],
+                                             uint32_t q0, uint32_t &bad, uint32_t &nonc) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const uint32_t le_n = lane_mask2(k0, i, 0, N), at_n = lane_mask2(k0, i, N, N);
+    const uint32_t e1 = __vsub2(__vsub2(__vadd2(qv[i], rv[i]), __vadd2(lo[i], mv[i])), (q0 | (q0 << 16)) & at_n);
+    const uint32_t e2 = __vadd2(qv[i], hi[i]) & lane_mask2(k0, i, 1, N);
+    bad |= (e1 & le_n | e2) & Q2;
+    nonc |= ((qv[i] | rv[i]) & ~Q2 & le_n) | (rv[i] & at_n);
+  }
+}
+
+// The same modulo 3 with byte witness arrays (qb, rb: 8 bytes).  The product coefficients are 16-bit residues of
+// c in (-2N, 4N): 65536 = 1 (mod 3), as in k_muldiv_imma.
+__device__ __forceinline__ void check_pass_3(int N, int k0, const uint32_t (&lo)[4], const uint32_t (&hi)[4], uint2 qb, uint2 rb,
+                                             uint32_t q0, uint32_t &bad, uint32_t &nonc) {
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int k = k0 + i;
+    const uint32_t lw = (lo[i >> 1] >> (16 * (i & 1))) & 0xffffu, hw = (hi[i >> 1] >> (16 * (i & 1))) & 0xffffu;
+    const uint32_t l3 = mod3_16(lw + (lw >> 15) * 2u), h3 = mod3_16(hw + (hw >> 15) * 2u);
+    const uint32_t qk = ((i < 4 ? qb.x : qb.y) >> (8 * (i & 3))) & 0xffu, rk = ((i < 4 ? rb.x : rb.y) >> (8 * (i & 3))) & 0xffu;
+    // -v = 2 v (mod 3): every term stays non-negative
+    const bool e1 = mod3_16(qk + rk + 2u * l3 + (k == N ? 2u * q0 : 0u)) != 0u;
+    const bool e2 = mod3_16(qk + h3) != 0u;
+    bad |= (k <= N && e1) || (k >= 1 && k <= N && e2);
+    nonc |= (k <= N && (qk >= 3u || rk >= 3u)) || (k == N && rk != 0u);
+  }
+}
+
+__device__ __forceinline__ void load_u16x8(const void *base, size_t off, bool act, uint32_t (&v)[4]) {
+  const uint4 t = act ? *reinterpret_cast<const uint4 *>(reinterpret_cast<const uint16_t *>(base) + off) : make_uint4(0, 0, 0, 0);
+  v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+}
+
+__device__ __forceinline__ uint2 load_u8x8(const void *base, size_t off, bool act) {
+  return act ? *reinterpret_cast<const uint2 *>(reinterpret_cast<const uint8_t *>(base) + off) : make_uint2(0, 0);
+}
+
+// Division modulo q of the product in cbuf against the uint16 witness (quo, rem) of `row`; m (encrypt) or nullptr.
+// Returns nonzero in bit 0 for a mismatch, bit 1 for a canonical-form violation (this lane's part).
+// R1 (decrypt): the lift b = (R1 + [R1 > q/2]) mod 3 of the raw witness remainder1 goes to xb.
+template <bool LIFT>
+__device__ __forceinline__ uint32_t check_div_q(int N, int P, uint32_t qmask, const uint16_t *cbuf, const void *quo, const void *rem,
+                                                const uint16_t *m, size_t row, int lane, uint8_t *xb) {
+  const uint32_t Q2 = qmask | (qmask << 16);
+  uint32_t bad = 0, nonc = 0, q0 = 0;
+  for (int kb = 0; kb < P; kb += 256) {
+    const int k0 = kb + 8 * lane;
+    const bool act = k0 < P;
+    const size_t off = row * (size_t)P + k0;
+    uint32_t lo[4] = {0, 0, 0, 0}, hi[4] = {0, 0, 0, 0}, qv[4], rv[4], mv[4] = {0, 0, 0, 0};
+    if (act) load_lo_hi2(N, cbuf, k0, lo, hi);
+    load_u16x8(quo, off, act, qv);
+    load_u16x8(rem, off, act, rv);
+    if (m) {
+      load_u16x8(m, off, act, mv);
+      mask_tail(mv, N - k0);          // m's pad columns are not part of the witness
+    }
+    if (kb == 0) q0 = __shfl_sync(0xffffffffu, qv[0], 0) & 0xffffu;
+    check_pass_q(N, k0, Q2, lo, hi, mv, qv, rv, q0, bad, nonc);
+    if (LIFT && act) {
+      const uint32_t half = (qmask + 1) >> 1;
+      uint32_t b[2] = {0u, 0u};
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const uint32_t r = (rv[i >> 1] >> (16 * (i & 1))) & 0xffffu;
+        b[i >> 2] |= (k0 + i < N ? mod3_16(r + (r > half ? 1u : 0u)) : 0u) << (8 * (i & 3));
+      }
+      *reinterpret_cast<uint2 *>(xb + k0) = make_uint2(b[0], b[1]);
+    }
+  }
+  return (bad ? 1u : 0u) | (nonc ? 2u : 0u);
+}
+
+__device__ __forceinline__ uint32_t check_div_3(int N, int P, const uint16_t *cbuf, const void *quo, const void *rem, size_t row, int lane) {
+  uint32_t bad = 0, nonc = 0, q0 = 0;
+  for (int kb = 0; kb < P; kb += 256) {
+    const int k0 = kb + 8 * lane;
+    const bool act = k0 < P;
+    const size_t off = row * (size_t)P + k0;
+    uint32_t lo[4] = {0, 0, 0, 0}, hi[4] = {0, 0, 0, 0};
+    if (act) load_lo_hi2(N, cbuf, k0, lo, hi);
+    const uint2 qb = load_u8x8(quo, off, act), rb = load_u8x8(rem, off, act);
+    if (kb == 0) q0 = __shfl_sync(0xffffffffu, qb.x, 0) & 0xffu;
+    if (act) check_pass_3(N, k0, lo, hi, qb, rb, q0, bad, nonc);
+  }
+  return (bad ? 1u : 0u) | (nonc ? 2u : 0u);
+}
+
+// the warp's verdict byte from every lane's domain flag and check bits
+__device__ __forceinline__ uint8_t check_verdict(bool domain_ok, uint32_t bits) {
+  const bool in_domain = __all_sync(0xffffffffu, domain_ok);
+  const bool sat = !__any_sync(0xffffffffu, bits & 1u);
+  const bool canon = sat && !__any_sync(0xffffffffu, bits & 2u);
+  return in_domain ? (uint8_t)((sat ? NTRU_CHECK_SATISFIED : 0) | (canon ? NTRU_CHECK_CANONICAL : 0)) : (uint8_t)NTRU_CHECK_DOMAIN;
+}
+
+// per-warp shared memory: the layout of the IMMA kernels (y0 | y1 | (y2) | xs | (xb) | cbuf), then the double-buffered
+// inputs [x : x_bytes][y : y_bytes][fp : P]; xs is the re-staged x behind kXPad zero bytes (the x6 slot)
+__host__ __device__ constexpr ImmaLayout make_check_layout(int N, int nj_bucket, bool dec, int in_bytes) {
+  ImmaLayout L = make_layout(N, nj_bucket, false, dec);
+  L.Lin = in_bytes;
+  L.warp_bytes = L.o_in + 2 * in_bytes;
+  return L;
+}
+
+#define NTRU_CHECK_PROLOGUE                                                                                               \
+  extern __shared__ __align__(16) uint8_t smem_raw[];                                                                    \
+  const ImmaLayout &L = a.L;                                                                                             \
+  const int N = L.N, P = L.P, Z = L.Z;                                                                                   \
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;                                                            \
+  uint8_t *base = smem_raw + (size_t)warp * L.warp_bytes;                                                                \
+  uint8_t *y0 = base, *y1 = base + L.o_y1, *y2 = base + L.o_y2, *xs = base + L.o_x6 + kXPad, *xb = base + L.o_xb + kXPad; \
+  uint16_t *cbuf = reinterpret_cast<uint16_t *>(base + L.o_c);                                                           \
+  uint8_t *in0 = base + L.o_in;                                                                                          \
+  for (int i = lane * 16; i < L.warp_bytes; i += 512) *reinterpret_cast<uint4 *>(base + i) = make_uint4(0, 0, 0, 0);     \
+  __syncwarp();                                                                                                          \
+  const size_t nwarps = (size_t)gridDim.x * kImmaWarps;                                                                  \
+  const uint32_t in_lane = (uint32_t)__cvta_generic_to_shared(in0) + 16 * lane;                                          \
+  (void)y2; (void)xb
+
+template <int NJ>
+__global__ void __launch_bounds__(kImmaWarps * 32) k_check_encrypt(const CheckArgs a) {
+  NTRU_CHECK_PROLOGUE;
+  auto prefetch = [&](size_t row, int buf) {
+    const uint32_t d = in_lane + buf * L.Lin;
+    prefetch_lane<0>(d, reinterpret_cast<const char *>(a.x) + (row * a.x_stride + 16 * lane), P, lane);
+    prefetch_lane<0>(d + P, reinterpret_cast<const char *>(a.y) + (row * a.y_stride * 2 + 16 * lane), 2 * P, lane);
+    prefetch_commit();
+  };
+  size_t row = (size_t)blockIdx.x * kImmaWarps + warp;
+  if (row < a.B) prefetch(row, 0);
+  int cur = 0;
+  for (; row < a.B; row += nwarps, cur ^= 1) {
+    uint8_t *in = in0 + cur * L.Lin;
+    uint8_t *xr = in, *yr = in + P;
+    prefetch_wait();
+    if (lane < P - N) reinterpret_cast<uint16_t *>(yr)[N + lane] = 0;      // the caller's pad columns may hold anything
+    __syncwarp();
+    stage_limbs<2, false>(N, Z, 0u, yr, y0, y1, lane);
+    const bool ok = stage_small<false>(N, P, a.M, xr, xs, lane);
+    __syncwarp();
+    if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);
+    {
+      int acc[NJ][2][4];
+      conv_band<NJ, 2, false, false, 0>(Z, y0, y1, xs, xs, lane, acc);
+      store_product<NJ, 2>(L.NJ, lane, acc, cbuf);
+    }
+    __syncwarp();
+    const uint32_t bits = check_div_q<false>(N, P, a.M - 1, cbuf, a.quo, a.rem, a.m, row, lane, nullptr);
+    const uint8_t v = check_verdict(ok, bits);
+    if (lane == 0) a.verdict[row] = v;
+    __syncwarp();
+  }
+}
+
+template <int NJ>
+__global__ void __launch_bounds__(kImmaWarps * 32) k_check_decrypt(const CheckArgs a) {
+  NTRU_CHECK_PROLOGUE;
+  auto prefetch = [&](size_t row, int buf) {
+    const uint32_t d = in_lane + buf * L.Lin;
+    prefetch_lane<0>(d, reinterpret_cast<const char *>(a.x) + (row * a.x_stride * 2 + 16 * lane), 2 * P, lane);
+    prefetch_lane<0>(d + 2 * P, reinterpret_cast<const char *>(a.y) + (row * a.y_stride * 2 + 16 * lane), 2 * P, lane);
+    prefetch_lane<0>(d + 4 * P, reinterpret_cast<const char *>(a.fp) + (row * a.x_stride + 16 * lane), P, lane);
+    prefetch_commit();
+  };
+  size_t row = (size_t)blockIdx.x * kImmaWarps + warp;
+  if (row < a.B) prefetch(row, 0);
+  int cur = 0;
+  for (; row < a.B; row += nwarps, cur ^= 1) {
+    uint8_t *in = in0 + cur * L.Lin;
+    uint8_t *fr = in, *er = in + 2 * P, *fpr = in + 4 * P;
+    prefetch_wait();
+    if (lane < P - N) {
+      reinterpret_cast<uint16_t *>(er)[N + lane] = 0;
+      fpr[N + lane] = 0;
+    }
+    __syncwarp();
+    stage_limbs<2, false>(N, Z, 0u, er, y0, y1, lane);
+    stage_rev8_mod3(N, Z, fpr, y2, lane);
+    const bool ok = stage_small<true>(N, P, a.M, fr, xs, lane);
+    __syncwarp();
+    if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);
+    {   // product 1: lin(f, e) mod q
+      int acc[NJ][2][4];
+      conv_band<NJ, 2, false, false, 0>(Z, y0, y1, xs, xs, lane, acc);
+      store_product<NJ, 2>(L.NJ, lane, acc, cbuf);
+    }
+    __syncwarp();
+    uint32_t bits = check_div_q<true>(N, P, a.M - 1, cbuf, a.quo, a.rem, nullptr, row, lane, xb);
+    __syncwarp();
+    {   // product 2: lin(fp mod 3, b), b in {0, 1, 2}: every coefficient in [0, 4N]
+      int acc[NJ][1][4];
+      conv_band<NJ, 1, false, false, 0>(Z, y2, y2, xb, xb, lane, acc);
+      store_product<NJ, 1>(L.NJ, lane, acc, cbuf);
+    }
+    __syncwarp();
+    bits |= check_div_3(N, P, cbuf, a.quo2, a.rem2, row, lane);
+    const uint8_t v = check_verdict(ok, bits);
+    if (lane == 0) a.verdict[row] = v;
+    __syncwarp();
+  }
+}
+
+template <int NJ, bool kModP>
+__global__ void __launch_bounds__(kImmaWarps * 32) k_check_inverse(const CheckArgs a) {
+  constexpr int LIMBS = kModP ? 1 : 2;
+  NTRU_CHECK_PROLOGUE;
+  const int ybytes = kModP ? P : 2 * P;
+  auto prefetch = [&](size_t row, int buf) {
+    const uint32_t d = in_lane + buf * L.Lin;
+    prefetch_lane<0>(d, reinterpret_cast<const char *>(a.x) + (row * (size_t)(2 * P) + 16 * lane), 2 * P, lane);
+    prefetch_lane<0>(d + 2 * P, reinterpret_cast<const char *>(a.y) + (row * (size_t)ybytes + 16 * lane), ybytes, lane);
+    prefetch_commit();
+  };
+  size_t row = (size_t)blockIdx.x * kImmaWarps + warp;
+  if (row < a.B) prefetch(row, 0);
+  int cur = 0;
+  for (; row < a.B; row += nwarps, cur ^= 1) {
+    uint8_t *in = in0 + cur * L.Lin;
+    uint8_t *xr = in, *yr = in + 2 * P;
+    prefetch_wait();
+    if (lane < P - N) {
+      if (kModP) yr[N + lane] = 0;
+      else reinterpret_cast<uint16_t *>(yr)[N + lane] = 0;
+    }
+    __syncwarp();
+    if (kModP) stage_rev8_mod3(N, Z, yr, y0, lane);
+    else stage_limbs<2, false>(N, Z, 0u, yr, y0, y1, lane);
+    const bool ok = stage_small<true>(N, P, a.M, xr, xs, lane);
+    __syncwarp();
+    if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);
+    {
+      int acc[NJ][LIMBS][4];
+      conv_band<NJ, LIMBS, false, false, 0>(Z, y0, y1, xs, xs, lane, acc);
+      store_product<NJ, LIMBS>(L.NJ, lane, acc, cbuf);
+    }
+    __syncwarp();
+    const uint32_t bits = kModP ? check_div_3(N, P, cbuf, a.quo, a.rem, row, lane)
+                                : check_div_q<false>(N, P, a.M - 1, cbuf, a.quo, a.rem, nullptr, row, lane, nullptr);
+    const uint8_t v = check_verdict(ok, bits);
+    if (lane == 0) a.verdict[row] = v;
+    __syncwarp();
+  }
+}
+
 template <class K, class A>
 int launch_imma(ntru_ctx *ctx, K kernel, const A &args, int kind, size_t B, int warp_bytes) {
   const size_t smem = (size_t)kImmaWarps * warp_bytes;
@@ -748,6 +1064,57 @@ int launch_decrypt_imma(ntru_ctx *ctx, size_t B, const int8_t *f, const uint8_t 
   a.B = B; a.f = f; a.fp = fp; a.key_stride = key_stride; a.e = e;
   a.value = value; a.q1 = q1; a.r1 = r1; a.q2 = q2; a.r2 = r2;
   NTRU_IMMA_DISPATCH(k_decrypt_imma, a, NTRU_K_DEC_IMMA);
+}
+
+// ---- witness checks: the generic instantiation of each N bucket ------------------------------------------------------
+#define NTRU_CHECK_DISPATCH(KERNEL, ...)                                                                          \
+  do {                                                                                                            \
+    const int nj = a.L.NJ, wb = a.L.warp_bytes;                                                                   \
+    if (nj <= 3) return launch_imma(ctx, KERNEL<3, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                       \
+    if (nj <= 8) return launch_imma(ctx, KERNEL<8, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                       \
+    if (nj <= 11) return launch_imma(ctx, KERNEL<11, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                     \
+    return launch_imma(ctx, KERNEL<13, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                                   \
+  } while (0)
+
+static int check_prologue(ntru_ctx *ctx, size_t B, CheckArgs &a, bool dec, int in_bytes, uint8_t *verdict) {
+  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "witness checks support N <= 832");
+  a = CheckArgs{};
+  a.L = make_check_layout(ctx->N, imma_bucket(ctx), dec, in_bytes);
+  a.M = (uint32_t)ctx->q;
+  a.B = B;
+  a.verdict = verdict;
+  return NTRU_OK;
+}
+
+int launch_check_encrypt(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t h_stride, const uint8_t *r, const uint16_t *m,
+                         const uint16_t *quo, const uint16_t *rem, uint8_t *verdict) {
+  if (B == 0) return NTRU_OK;
+  const size_t P = (size_t)ctx->P;
+  CheckArgs a;
+  if (int rc = check_prologue(ctx, B, a, false, 3 * ctx->P, verdict)) return rc;
+  a.x = r; a.x_stride = P; a.y = h; a.y_stride = h_stride; a.m = m; a.quo = quo; a.rem = rem;
+  NTRU_CHECK_DISPATCH(k_check_encrypt);
+}
+
+int launch_check_decrypt(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, size_t key_stride, const uint16_t *e,
+                         const uint16_t *q1, const uint16_t *r1, const uint8_t *q2, const uint8_t *r2, uint8_t *verdict) {
+  if (B == 0) return NTRU_OK;
+  CheckArgs a;
+  if (int rc = check_prologue(ctx, B, a, true, 5 * ctx->P, verdict)) return rc;
+  a.x = f; a.fp = fp; a.x_stride = key_stride; a.y = e; a.y_stride = (size_t)ctx->P;
+  a.quo = q1; a.rem = r1; a.quo2 = q2; a.rem2 = r2;
+  NTRU_CHECK_DISPATCH(k_check_decrypt);
+}
+
+int launch_check_inverse(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y, const void *quo, const void *rem,
+                         uint8_t *verdict) {
+  if (B == 0) return NTRU_OK;
+  CheckArgs a;
+  if (int rc = check_prologue(ctx, B, a, false, (mod_p ? 3 : 4) * ctx->P, verdict)) return rc;
+  if (mod_p) a.M = (uint32_t)ctx->p;
+  a.x = x; a.y = y; a.quo = quo; a.rem = rem;
+  if (mod_p) NTRU_CHECK_DISPATCH(k_check_inverse, true);
+  NTRU_CHECK_DISPATCH(k_check_inverse, false);
 }
 
 }  // namespace ntru

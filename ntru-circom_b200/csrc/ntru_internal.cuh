@@ -64,6 +64,7 @@ struct ntru_ctx {
   ntru::DevBuf slot_packed[ntru::kNumSlots][10];   // packed staging (what the 1-D H2D / D2H copies move)
   ntru::DevBuf d_partial;
   ntru::DevBuf kg_bufs[12];         // key generation: lifting scratch (t, u0, u1, r0, r1), host-form rows, valid, count
+  ntru::DevBuf check_key[2];       // witness checks, host form: the shared key row (h, or f and fp)
   ntru::DevBuf d_sum_scratch;      // tree scratch of the ciphertext sum (per-CTA rows, per-group rows, tickets)
   // cross-GPU sum: exchange window (this rank's, cudaMalloc + IPC) and the mapped windows of the peers
   static constexpr int kMaxRanks = 16;
@@ -165,6 +166,14 @@ int launch_decrypt_imma(ntru_ctx *ctx, size_t B, const int8_t *f, const uint8_t 
                         uint8_t *value, uint16_t *q1, uint16_t *r1, uint8_t *q2, uint8_t *r2);
 
 int launch_muldiv_imma(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int mod_p, void *quo, void *rem);
+
+// witness checks (VerifyEncrypt / VerifyDecrypt / VerifyInverse) on the same product, one verdict byte per row
+int launch_check_encrypt(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t h_stride, const uint8_t *r, const uint16_t *m,
+                         const uint16_t *quo, const uint16_t *rem, uint8_t *verdict);
+int launch_check_decrypt(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, size_t key_stride, const uint16_t *e,
+                         const uint16_t *q1, const uint16_t *r1, const uint8_t *q2, const uint8_t *r2, uint8_t *verdict);
+int launch_check_inverse(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y, const void *quo, const void *rem,
+                         uint8_t *verdict);
 
 // ---- batched key generation (keygen.cu): divstep inversions modulo 2 and 3, IMMA lifting to q and h ----
 constexpr int kKeygenRounds = 100;   // draws of f per key before giving up (index.js:52-64)

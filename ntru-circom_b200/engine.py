@@ -290,6 +290,78 @@ class Engine:
         """multiplyPolynomials(x, y, mod) + dividePolynomials(., 1 - x^N, mod), device-resident rows."""
         self._check(self.lib.ntru_muldiv_dev(self._h, B, _ptr(x), _ptr(y), int(bool(mod_p)), _ptr(quotient), _ptr(remainder)))
 
+    # -- witness checks: VerifyEncrypt / VerifyDecrypt / VerifyInverse (ntru.circom:155-256), one verdict byte per row ------
+    def _key(self, a, dtype, B):
+        """A key array of a check: (N,) is one row shared by every witness, (B, N) one row per witness."""
+        a = np.asarray(a)
+        shared = a.ndim == 1
+        return _host(a, dtype, (self.N,) if shared else (B, self.N)), shared
+
+    def check_encrypt(self, h, r, m, quotientE, remainderE):
+        """Verdicts (B,) uint8 of NTRU_CHECK_* bits for B VerifyEncrypt witnesses: r (B, N) bytes, m (B, N) uint16,
+        quotientE / remainderE (B, N + 1) uint16; h (N,) shared or (B, N)."""
+        N = self.N
+        r = np.asarray(r)
+        B = r.shape[0]
+        h, shared = self._key(h, np.uint16, B)
+        r = _host(r, np.uint8, (B, N))
+        m = _host(m, np.uint16, (B, N))
+        quo = _host(quotientE, np.uint16, (B, N + 1))
+        rem = _host(remainderE, np.uint16, (B, N + 1))
+        verdict = np.empty(B, dtype=np.uint8)
+        self._check(self.lib.ntru_check_encrypt_batch(self._h, B, _ptr(h), int(shared), _ptr(r), _ptr(m), _ptr(quo), _ptr(rem),
+                                                      _ptr(verdict)))
+        return verdict
+
+    def check_decrypt(self, f, fp, e, quotient1, remainder1, quotient2, remainder2):
+        """Verdicts for B VerifyDecrypt witnesses: f (uint16, -1 as q - 1) and fp (bytes), both (N,) shared or (B, N);
+        e (B, N) uint16; quotient1 / remainder1 (B, N + 1) uint16, quotient2 / remainder2 (B, N + 1) bytes."""
+        N = self.N
+        e = np.asarray(e)
+        B = e.shape[0]
+        f, shared = self._key(f, np.uint16, B)
+        fp, fp_shared = self._key(fp, np.uint8, B)
+        if shared != fp_shared:
+            raise ValueError("f and fp must both be one shared row or both be one row per witness")
+        e = _host(e, np.uint16, (B, N))
+        q1 = _host(quotient1, np.uint16, (B, N + 1))
+        r1 = _host(remainder1, np.uint16, (B, N + 1))
+        q2 = _host(quotient2, np.uint8, (B, N + 1))
+        r2 = _host(remainder2, np.uint8, (B, N + 1))
+        verdict = np.empty(B, dtype=np.uint8)
+        self._check(self.lib.ntru_check_decrypt_batch(self._h, B, _ptr(f), _ptr(fp), int(shared), _ptr(e), _ptr(q1), _ptr(r1),
+                                                      _ptr(q2), _ptr(r2), _ptr(verdict)))
+        return verdict
+
+    def check_inverse(self, x, y, quotientI, remainderI, mod_p=False):
+        """Verdicts for B VerifyInverse witnesses: x (B, N) uint16; modulo q, y (B, N) and quotientI / remainderI
+        (B, N + 1) uint16; modulo p (mod_p=True, the fp case) the same as bytes."""
+        N = self.N
+        x = np.asarray(x)
+        B = x.shape[0]
+        t = np.uint8 if mod_p else np.uint16
+        x = _host(x, np.uint16, (B, N))
+        y = _host(y, t, (B, N))
+        quo = _host(quotientI, t, (B, N + 1))
+        rem = _host(remainderI, t, (B, N + 1))
+        verdict = np.empty(B, dtype=np.uint8)
+        self._check(self.lib.ntru_check_inverse_batch(self._h, B, int(bool(mod_p)), _ptr(x), _ptr(y), _ptr(quo), _ptr(rem),
+                                                      _ptr(verdict)))
+        return verdict
+
+    def check_encrypt_dev(self, B, h, key_stride, r, m, quotientE, remainderE, verdict):
+        """check_encrypt on device rows (pitch self.pitch), asynchronous; key_stride 0 (one h row) or self.pitch."""
+        self._check(self.lib.ntru_check_encrypt_dev(self._h, B, _ptr(h), int(key_stride), _ptr(r), _ptr(m), _ptr(quotientE),
+                                                    _ptr(remainderE), _ptr(verdict)))
+
+    def check_decrypt_dev(self, B, f, fp, key_stride, e, quotient1, remainder1, quotient2, remainder2, verdict):
+        self._check(self.lib.ntru_check_decrypt_dev(self._h, B, _ptr(f), _ptr(fp), int(key_stride), _ptr(e), _ptr(quotient1),
+                                                    _ptr(remainder1), _ptr(quotient2), _ptr(remainder2), _ptr(verdict)))
+
+    def check_inverse_dev(self, B, mod_p, x, y, quotientI, remainderI, verdict):
+        self._check(self.lib.ntru_check_inverse_dev(self._h, B, int(bool(mod_p)), _ptr(x), _ptr(y), _ptr(quotientI),
+                                                    _ptr(remainderI), _ptr(verdict)))
+
     # -- packOutput / unpackInput (index.js:572-620) on device rows --------------------------------------
     def pack_geometry(self, max_val: int, data_len: int):
         v = [ctypes.c_int() for _ in range(4)]

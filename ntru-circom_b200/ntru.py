@@ -346,6 +346,33 @@ class NTRU:
                              "quotientI": ex(hDiv["quotient"], N + 1, 0), "remainderI": ex(hDiv["remainder"], N + 1, 0)}},
         }
 
+    # ---- witness checks: the circuits' constraint systems (ntru.circom:155-256) for many witnesses at once ------------
+    def _check_params(self, params, want, what):
+        got = [int(x) for x in params]
+        if got != want:
+            raise ValueError(f"{what} params {got} do not match this instance's {want}")
+
+    def verifyEncryptBatch(self, inputs: dict, params) -> np.ndarray:
+        """VerifyEncrypt for B witnesses: inputs under the reference's names (r, m, h, quotientE, remainderE), each
+        (B, width); h may be one (N,) row.  Returns the uint8 verdicts (NTRU_CHECK_SATISFIED | _CANONICAL | _DOMAIN)."""
+        self._check_params(params, [self.q, self.calculateNq(), self.N], "VerifyEncrypt")
+        return self.engine().check_encrypt(inputs["h"], inputs["r"], inputs["m"], inputs["quotientE"], inputs["remainderE"])
+
+    def verifyDecryptBatch(self, inputs: dict, params) -> np.ndarray:
+        """VerifyDecrypt for B witnesses (f, fp, e, quotient1, remainder1, quotient2, remainder2); f and fp may be one
+        (N,) row each."""
+        self._check_params(params, [self.q, self.calculateNq(), self.p, self.calculateNp(), self.N], "VerifyDecrypt")
+        return self.engine().check_decrypt(inputs["f"], inputs["fp"], inputs["e"], inputs["quotient1"], inputs["remainder1"],
+                                           inputs["quotient2"], inputs["remainder2"])
+
+    def verifyInverseBatch(self, inputs: dict, params) -> np.ndarray:
+        """VerifyInverse for B witnesses (f, fq, quotientI, remainderI) as verifyKeysInputs emits them; params[0] picks the
+        case: q (the fq and h cases) or p (the fp case)."""
+        mod_p = len(params) > 0 and int(params[0]) == self.p
+        want = [self.p, self.calculateNp(), self.N] if mod_p else [self.q, self.calculateNq(), self.N]
+        self._check_params(params, want, "VerifyInverse")
+        return self.engine().check_inverse(inputs["f"], inputs["fq"], inputs["quotientI"], inputs["remainderI"], mod_p=mod_p)
+
     # ---- index.js:201-206 ----------------------------------------------------------------
     def calculateNq(self) -> int:
         return math.ceil(math.log2(self.q * self.q * self.N))
