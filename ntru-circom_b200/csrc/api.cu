@@ -603,11 +603,6 @@ int ntru_decrypt_batch_packed(ntru_ctx *ctx, size_t B, const void *e, void *valu
                       (uint8_t *)quotient2, (uint8_t *)remainder2, true);
 }
 
-__global__ void k_scale_u16(const uint16_t *__restrict__ src, uint16_t *__restrict__ dst, size_t n, uint32_t mul) {
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-    dst[i] = (uint16_t)(src[i] * mul);
-}
-
 int ntru_muldiv_dev(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int mod_p, void *quotient, void *remainder) {
   int rc = check(ctx);
   if (rc) return rc;
@@ -643,17 +638,8 @@ int ntru_verify_keys_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const uint1
     // fp case: x = f (the value p-1 of a -1 is the same residue), y = fp
     if (dev[6] || dev[7]) r2 = launch_muldiv_imma(ctx, rows, (const int8_t *)dev[0], dev[2], 1, dev[6], dev[7]);
     if (r2) return r2;
-    if (dev[8] || dev[9]) {
-      // h case: y = p * fq, NOT reduced mod q (index.js:155); 3 * (q - 1) < 65536 for q <= 16384
-      NTRU_CUDA(ctx, ctx->d_b.reserve(rows * (size_t)ctx->P * 2));
-      {
-        LaunchTimer timer(ctx, NTRU_K_OTHER);
-        k_scale_u16<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>((const uint16_t *)dev[1], (uint16_t *)ctx->d_b.ptr,
-                                                               rows * (size_t)ctx->P, (uint32_t)ctx->p);
-      }
-      NTRU_CUDA(ctx, cudaGetLastError());
-      r2 = launch_muldiv_imma(ctx, rows, (const int8_t *)dev[3], ctx->d_b.ptr, 0, dev[8], dev[9]);
-    }
+    if (dev[8] || dev[9])
+      r2 = launch_h_product(ctx, rows, (const int8_t *)dev[3], (const uint16_t *)dev[1], (uint16_t *)dev[8], (uint16_t *)dev[9]);
     return r2;
   });
 }

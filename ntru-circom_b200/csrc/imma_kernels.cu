@@ -30,6 +30,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "ntru_internal.cuh"
 
 namespace ntru {
@@ -54,6 +56,10 @@ __device__ __forceinline__ void imma_u8u8(int (&c)[4], const uint32_t (&a)[4], u
 __device__ __forceinline__ uint32_t mod3_16(uint32_t v) {   // two instructions: floor(v / 3) = umulhi(v, (2^32 + 2) / 3) for v < 2^31
   return v - 3u * __umulhi(v, 0x55555556u);
 }
+
+// residue mod 3 of a product coefficient c in (-2N, 4N) (x may hold -1) from its 16-bit word w = c mod 65536:
+// 65536 = 1 (mod 3), so the representative c + 65536 of a negative c is 1 too high, and adding 2 removes that
+__device__ __forceinline__ uint32_t mod3_prod16(uint32_t w) { return mod3_16(w + (w >> 15) * 2u); }
 
 // Column blocks visited per K step: jn = (s >> 2) + d, d = 0 .. kDMax.  Some K1 - t of block (jn, s) lies in [0, I1)
 // iff  s >> 2 <= jn <= (2 s + I1) >> 3; with I1 <= 4 NJ that is d <= (6 + 4 NJ) >> 3.  The few visited blocks outside
@@ -184,14 +190,15 @@ __device__ __forceinline__ void store_product(int nj, int lane, const int (&acc)
 //   y0, y1  reversed limb arrays of h (encrypt) or e (decrypt); y2 reversed fp (decrypt)
 //   x6      64 x behind kXPad zero bytes (x = r or f); xb the lifted polynomial b of decrypt, same shape
 //   cbuf    the 2N - 1 product coefficients mod 2^16
-//   in[2]   the row's inputs as cp.async delivers them, double buffered: [kXPad zeros | x : P | zeros up to Lx] [y : 2P] [m or fp : P]
-//           -- the x part is laid out so that the B fragments of the low limb are read from it in place.
+//   in[2]   the row's inputs as cp.async delivers them, double buffered, in_bytes each; in_bytes = 0: the encrypt / decrypt
+//           form [kXPad zeros | x : P | zeros up to Lx] [y : 2P] [m or fp : P], laid out so that the B fragments of the
+//           low limb are read from the x part in place
 struct ImmaLayout {
   int N, P, I1, S, NJ, Z, Ly, Lx, Lc, Lin;
   int o_y1, o_y2, o_x6, o_xb, o_c, o_in, warp_bytes;
 };
 
-__host__ __device__ constexpr ImmaLayout make_layout(int N, int nj_bucket, bool exact, bool dec) {
+__host__ __device__ constexpr ImmaLayout make_layout(int N, int nj_bucket, bool exact, bool dec, int in_bytes) {
   ImmaLayout L{};
   L.N = N;
   L.P = ((N + 1 + 15) / 16) * 16;
@@ -207,7 +214,7 @@ __host__ __device__ constexpr ImmaLayout make_layout(int N, int nj_bucket, bool 
   const int dmax = (6 + 4 * nj_bucket) >> 3;
   L.Lx = kXPad + (128 * (dmax + 1) > L.P ? 128 * (dmax + 1) : L.P);
   L.Lc = 2 * (128 * L.NJ + 32);
-  L.Lin = L.Lx + 3 * L.P;
+  L.Lin = in_bytes ? in_bytes : L.Lx + 3 * L.P;
   int o = L.Ly;
   L.o_y1 = o; o += L.Ly;
   L.o_y2 = o; if (dec) o += L.Ly;
@@ -237,13 +244,26 @@ __device__ __forceinline__ void stage_limbs(int N, int Z, uint32_t Q2, const uin
   }
 }
 
-// bytes -> reversed array
+// bytes -> reversed array; MOD3: every byte reduced modulo 3 on the way.  The copy is unrolled twice; the mod-3 form,
+// four times the instructions per step, is not unrolled (the compiler's choice for it before the two were merged,
+// pinned here so that either form keeps its code)
+template <bool MOD3>
 __device__ __forceinline__ void stage_rev8(int N, int Z, const uint8_t *src, uint8_t *y, int lane) {
-#pragma unroll 2
+#pragma unroll (MOD3 ? 1 : 2)
   for (int j0 = 16 * lane; j0 < N; j0 += 512) {
     const uint4 v = *reinterpret_cast<const uint4 *>(src + j0);
+    uint32_t w[4] = {v.x, v.y, v.z, v.w};
+    if (MOD3) {
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        uint32_t o = 0;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) o |= mod3_16((w[i] >> (8 * b)) & 0xffu) << (8 * b);
+        w[i] = o;
+      }
+    }
     *reinterpret_cast<uint4 *>(y + (Z - j0 - 15)) =
-        make_uint4(__byte_perm(v.w, 0u, 0x0123), __byte_perm(v.z, 0u, 0x0123), __byte_perm(v.y, 0u, 0x0123), __byte_perm(v.x, 0u, 0x0123));
+        make_uint4(__byte_perm(w[3], 0u, 0x0123), __byte_perm(w[2], 0u, 0x0123), __byte_perm(w[1], 0u, 0x0123), __byte_perm(w[0], 0u, 0x0123));
   }
 }
 
@@ -309,6 +329,16 @@ __device__ __forceinline__ void prefetch_lane(uint32_t dst, const char *src, int
   }
 }
 
+// division by 1 - x^N modulo q (Q2 = q - 1 in both lanes) of 8 packed coefficients: remainder lo + hi, quotient -hi
+__device__ __forceinline__ void div_xn_q(uint32_t Q2, const uint32_t (&lo)[4], const uint32_t (&hi)[4], uint32_t (&rem)[4],
+                                         uint32_t (&quo)[4]) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    rem[i] = __vadd2(lo[i], hi[i]) & Q2;
+    quo[i] = __vsub2(0u, hi[i]) & Q2;
+  }
+}
+
 // zeroes the packed uint16 lanes k0 + i >= N of an 8-coefficient vector (branch-free)
 __device__ __forceinline__ void mask_tail(uint32_t (&v)[4], int nv) {
 #pragma unroll
@@ -331,7 +361,7 @@ struct ImmaEncArgs {
 template <int NJ, int LIMBS, int NX>
 __global__ void __launch_bounds__(kImmaWarps * 32, ImmaShape<NJ>::kMinBlocks) k_encrypt_imma(const ImmaEncArgs a) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
-  constexpr ImmaLayout LX = make_layout(NX ? NX : 16, NJ, true, false);
+  constexpr ImmaLayout LX = make_layout(NX ? NX : 16, NJ, true, false, 0);
   constexpr int I1X = NX ? (NX + 15) / 16 : 0;
   const int N = NTRU_LF(N), P = NTRU_LF(P), Z = NTRU_LF(Z), Lx = NTRU_LF(Lx), Lin = NTRU_LF(Lin);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -422,7 +452,7 @@ struct ImmaDecArgs {
 template <int NJ, int LIMBS, int NX>
 __global__ void __launch_bounds__(kImmaWarps * 32, ImmaShape<NJ>::kMinBlocks) k_decrypt_imma(const ImmaDecArgs a) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
-  constexpr ImmaLayout LX = make_layout(NX ? NX : 16, NJ, true, true);
+  constexpr ImmaLayout LX = make_layout(NX ? NX : 16, NJ, true, true, 0);
   constexpr int I1X = NX ? (NX + 15) / 16 : 0;
   const int N = NTRU_LF(N), P = NTRU_LF(P), Z = NTRU_LF(Z), Lx = NTRU_LF(Lx), Lin = NTRU_LF(Lin);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -461,7 +491,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32, ImmaShape<NJ>::kMinBlocks) k_
     __syncwarp();
     stage_limbs<LIMBS, true>(N, Z, Q2, er, y0, y1, lane);
     if (LIMBS == 2) stage_x6(N, fr, x6 + kXPad, lane);
-    stage_rev8(N, Z, fpr, y2, lane);
+    stage_rev8<false>(N, Z, fpr, y2, lane);
     __syncwarp();
     if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);    // in flight during this row's products
     {   // product 1: a = lin(f, e) mod q  (f in {-1, 0, 1}: signed multiplier)
@@ -478,11 +508,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32, ImmaShape<NJ>::kMinBlocks) k_
         if (kb < P && (kb + 256 <= P || k0 < P)) {
           uint32_t lo[4], hi[4], rem[4], quo[4];
           load_lo_hi2(N, cbuf, k0, lo, hi);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            rem[i] = __vadd2(lo[i], hi[i]) & Q2;
-            quo[i] = __vsub2(0u, hi[i]) & Q2;
-          }
+          div_xn_q(Q2, lo, hi, rem, quo);
           if (kb + 256 > N) {       // only the last pass holds columns beyond N
             mask_tail(rem, N - k0);
             mask_tail(quo, N - k0);
@@ -587,7 +613,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_muldiv_imma(const ImmaMulDi
       else reinterpret_cast<uint16_t *>(yr)[N + lane] = 0;
     }
     __syncwarp();
-    if (kModP) stage_rev8(N, Z, yr, y0, lane);
+    if (kModP) stage_rev8<false>(N, Z, yr, y0, lane);
     else stage_limbs<2, false>(N, Z, Q2, yr, y0, y1, lane);
     __syncwarp();
     if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);
@@ -618,11 +644,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_muldiv_imma(const ImmaMulDi
         if (a.quo) *reinterpret_cast<uint2 *>(reinterpret_cast<uint8_t *>(a.quo) + rbase + k0) = make_uint2(quo[0], quo[1]);
       } else {
         uint32_t rem[4], quo[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          rem[i] = __vadd2(lo[i], hi[i]) & Q2;
-          quo[i] = __vsub2(0u, hi[i]) & Q2;
-        }
+        div_xn_q(Q2, lo, hi, rem, quo);
         mask_tail(rem, N - k0);
         mask_tail(quo, N - k0);
         if (a.rem) *reinterpret_cast<uint4 *>(reinterpret_cast<uint16_t *>(a.rem) + rbase + k0) = make_uint4(rem[0], rem[1], rem[2], rem[3]);
@@ -676,23 +698,6 @@ __device__ __forceinline__ bool stage_small(int N, int P, uint32_t M, const uint
   return ok;
 }
 
-// bytes -> reversed array, every byte reduced modulo 3 (stage_rev8 copies them as they are)
-__device__ __forceinline__ void stage_rev8_mod3(int N, int Z, const uint8_t *src, uint8_t *y, int lane) {
-  for (int j0 = 16 * lane; j0 < N; j0 += 512) {
-    const uint4 v = *reinterpret_cast<const uint4 *>(src + j0);
-    uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      uint32_t o = 0;
-#pragma unroll
-      for (int b = 0; b < 4; ++b) o |= mod3_16((w[i] >> (8 * b)) & 0xffu) << (8 * b);
-      w[i] = o;
-    }
-    *reinterpret_cast<uint4 *>(y + (Z - j0 - 15)) =
-        make_uint4(__byte_perm(w[3], 0u, 0x0123), __byte_perm(w[2], 0u, 0x0123), __byte_perm(w[1], 0u, 0x0123), __byte_perm(w[0], 0u, 0x0123));
-  }
-}
-
 // packed uint16 lanes of the 8 coefficients k0 .. k0+7 with lo_k <= k <= hi_k
 __device__ __forceinline__ uint32_t lane_mask2(int k0, int i, int lo_k, int hi_k) {
   const int k = k0 + 2 * i;
@@ -715,14 +720,14 @@ __device__ __forceinline__ void check_pass_q(int N, int k0, uint32_t Q2, const u
 }
 
 // The same modulo 3 with byte witness arrays (qb, rb: 8 bytes).  The product coefficients are 16-bit residues of
-// c in (-2N, 4N): 65536 = 1 (mod 3), as in k_muldiv_imma.
+// c in (-2N, 4N), as in k_muldiv_imma.
 __device__ __forceinline__ void check_pass_3(int N, int k0, const uint32_t (&lo)[4], const uint32_t (&hi)[4], uint2 qb, uint2 rb,
                                              uint32_t q0, uint32_t &bad, uint32_t &nonc) {
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int k = k0 + i;
     const uint32_t lw = (lo[i >> 1] >> (16 * (i & 1))) & 0xffffu, hw = (hi[i >> 1] >> (16 * (i & 1))) & 0xffffu;
-    const uint32_t l3 = mod3_16(lw + (lw >> 15) * 2u), h3 = mod3_16(hw + (hw >> 15) * 2u);
+    const uint32_t l3 = mod3_prod16(lw), h3 = mod3_prod16(hw);
     const uint32_t qk = ((i < 4 ? qb.x : qb.y) >> (8 * (i & 3))) & 0xffu, rk = ((i < 4 ? rb.x : rb.y) >> (8 * (i & 3))) & 0xffu;
     // -v = 2 v (mod 3): every term stays non-negative
     const bool e1 = mod3_16(qk + rk + 2u * l3 + (k == N ? 2u * q0 : 0u)) != 0u;
@@ -802,13 +807,6 @@ __device__ __forceinline__ uint8_t check_verdict(bool domain_ok, uint32_t bits) 
 
 // per-warp shared memory: the layout of the IMMA kernels (y0 | y1 | (y2) | xs | (xb) | cbuf), then the double-buffered
 // inputs [x : x_bytes][y : y_bytes][fp : P]; xs is the re-staged x behind kXPad zero bytes (the x6 slot)
-__host__ __device__ constexpr ImmaLayout make_check_layout(int N, int nj_bucket, bool dec, int in_bytes) {
-  ImmaLayout L = make_layout(N, nj_bucket, false, dec);
-  L.Lin = in_bytes;
-  L.warp_bytes = L.o_in + 2 * in_bytes;
-  return L;
-}
-
 #define NTRU_CHECK_PROLOGUE                                                                                               \
   extern __shared__ __align__(16) uint8_t smem_raw[];                                                                    \
   const ImmaLayout &L = a.L;                                                                                             \
@@ -882,7 +880,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_check_decrypt(const CheckAr
     }
     __syncwarp();
     stage_limbs<2, false>(N, Z, 0u, er, y0, y1, lane);
-    stage_rev8_mod3(N, Z, fpr, y2, lane);
+    stage_rev8<true>(N, Z, fpr, y2, lane);
     const bool ok = stage_small<true>(N, P, a.M, fr, xs, lane);
     __syncwarp();
     if (row + nwarps < a.B) prefetch(row + nwarps, cur ^ 1);
@@ -930,7 +928,7 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_check_inverse(const CheckAr
       else reinterpret_cast<uint16_t *>(yr)[N + lane] = 0;
     }
     __syncwarp();
-    if (kModP) stage_rev8_mod3(N, Z, yr, y0, lane);
+    if (kModP) stage_rev8<true>(N, Z, yr, y0, lane);
     else stage_limbs<2, false>(N, Z, 0u, yr, y0, y1, lane);
     const bool ok = stage_small<true>(N, P, a.M, xr, xs, lane);
     __syncwarp();
@@ -949,9 +947,13 @@ __global__ void __launch_bounds__(kImmaWarps * 32) k_check_inverse(const CheckAr
   }
 }
 
+// every launch of this file: nothing to do for B = 0, an error for N or q beyond the schedule
 template <class K, class A>
-int launch_imma(ntru_ctx *ctx, K kernel, const A &args, int kind, size_t B, int warp_bytes) {
-  const size_t smem = (size_t)kImmaWarps * warp_bytes;
+int launch_imma(ntru_ctx *ctx, K kernel, const A &args, int kind) {
+  const size_t B = args.B;
+  if (B == 0) return NTRU_OK;
+  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "register-fragment tensor schedule supports N <= 832");
+  const size_t smem = (size_t)kImmaWarps * args.L.warp_bytes;
   // occupancy: once per (context, kernel, footprint), not per launch
   int per_sm = 0;
   for (const auto &c : ctx->imma_cfg)
@@ -1005,116 +1007,100 @@ static int imma_exact_n(const ntru_ctx *ctx) {
   }
 }
 
-#define NTRU_IMMA_DISPATCH(KERNEL, ARGS, KIND)                                                        \
-  do {                                                                                                \
-    const int nj = (ARGS).L.NJ, wb = (ARGS).L.warp_bytes;                                             \
-    const bool two = ctx->q > 256;                                                                    \
-    switch (imma_exact_n(ctx)) {                                                                      \
-      case 167: return launch_imma(ctx, KERNEL<3, 1, 167>, ARGS, KIND, B, wb);                        \
-      case 509: return launch_imma(ctx, KERNEL<8, 2, 509>, ARGS, KIND, B, wb);                        \
-      case 677: return launch_imma(ctx, KERNEL<11, 2, 677>, ARGS, KIND, B, wb);                       \
-      case 701: return launch_imma(ctx, KERNEL<11, 2, 701>, ARGS, KIND, B, wb);                       \
-      case 821: return launch_imma(ctx, KERNEL<13, 2, 821>, ARGS, KIND, B, wb);                       \
-      default: break;                                                                                 \
-    }                                                                                                 \
-    if (nj <= 3) return two ? launch_imma(ctx, KERNEL<3, 2, 0>, ARGS, KIND, B, wb) : launch_imma(ctx, KERNEL<3, 1, 0>, ARGS, KIND, B, wb);   \
-    if (nj <= 8) return two ? launch_imma(ctx, KERNEL<8, 2, 0>, ARGS, KIND, B, wb) : launch_imma(ctx, KERNEL<8, 1, 0>, ARGS, KIND, B, wb);   \
-    if (nj <= 11) return two ? launch_imma(ctx, KERNEL<11, 2, 0>, ARGS, KIND, B, wb) : launch_imma(ctx, KERNEL<11, 1, 0>, ARGS, KIND, B, wb); \
-    return two ? launch_imma(ctx, KERNEL<13, 2, 0>, ARGS, KIND, B, wb) : launch_imma(ctx, KERNEL<13, 1, 0>, ARGS, KIND, B, wb);              \
-  } while (0)
+template <int V> using Int = std::integral_constant<int, V>;
+
+// launch(Int<NJ>{}) for the N bucket of ctx: the generic instantiation of NJ column blocks
+template <class F>
+static int for_bucket(const ntru_ctx *ctx, F launch) {
+  switch (imma_bucket(ctx)) {
+    case 3: return launch(Int<3>{});
+    case 8: return launch(Int<8>{});
+    case 11: return launch(Int<11>{});
+    default: return launch(Int<13>{});
+  }
+}
+
+// encrypt / decrypt: launch(Int<NJ>{}, Int<LIMBS>{}, Int<NX>{}) for the instantiation that serves ctx
+template <class F>
+static int for_enc_dec_form(const ntru_ctx *ctx, F launch) {
+  switch (imma_exact_n(ctx)) {
+    case 167: return launch(Int<3>{}, Int<1>{}, Int<167>{});
+    case 509: return launch(Int<8>{}, Int<2>{}, Int<509>{});
+    case 677: return launch(Int<11>{}, Int<2>{}, Int<677>{});
+    case 701: return launch(Int<11>{}, Int<2>{}, Int<701>{});
+    case 821: return launch(Int<13>{}, Int<2>{}, Int<821>{});
+    default: break;
+  }
+  const bool two = ctx->q > 256;
+  return for_bucket(ctx, [&](auto nj) { return two ? launch(nj, Int<2>{}, Int<0>{}) : launch(nj, Int<1>{}, Int<0>{}); });
+}
 
 int launch_muldiv_imma(ntru_ctx *ctx, size_t B, const int8_t *x, const void *y, int mod_p, void *quo, void *rem) {
-  if (B == 0) return NTRU_OK;
-  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "register-fragment tensor schedule supports N <= 832");
   ImmaMulDivArgs a;
-  a.L = make_layout(ctx->N, imma_bucket(ctx), false, false);
+  a.L = make_layout(ctx->N, imma_bucket(ctx), false, false, 0);
   a.qmask = (uint32_t)ctx->q - 1;
   a.B = B; a.x = x; a.y = y; a.quo = quo; a.rem = rem;
-  const int nj = a.L.NJ;
-  if (mod_p) {
-    if (nj <= 3) return launch_imma(ctx, k_muldiv_imma<3, true>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-    if (nj <= 8) return launch_imma(ctx, k_muldiv_imma<8, true>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-    if (nj <= 11) return launch_imma(ctx, k_muldiv_imma<11, true>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-    return launch_imma(ctx, k_muldiv_imma<13, true>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-  }
-  if (nj <= 3) return launch_imma(ctx, k_muldiv_imma<3, false>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-  if (nj <= 8) return launch_imma(ctx, k_muldiv_imma<8, false>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-  if (nj <= 11) return launch_imma(ctx, k_muldiv_imma<11, false>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
-  return launch_imma(ctx, k_muldiv_imma<13, false>, a, NTRU_K_MULDIV, B, a.L.warp_bytes);
+  return for_bucket(ctx, [&](auto nj) {
+    return mod_p ? launch_imma(ctx, k_muldiv_imma<nj, true>, a, NTRU_K_MULDIV) : launch_imma(ctx, k_muldiv_imma<nj, false>, a, NTRU_K_MULDIV);
+  });
 }
 
 int launch_encrypt_imma(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t h_stride, const uint8_t *r, const uint8_t *m,
                         uint16_t *value, uint16_t *quo, uint16_t *rem) {
-  if (B == 0) return NTRU_OK;
-  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "register-fragment tensor schedule supports N <= 832");
   ImmaEncArgs a;
-  a.L = make_layout(ctx->N, imma_bucket(ctx), imma_exact_n(ctx) != 0, false);
+  a.L = make_layout(ctx->N, imma_bucket(ctx), imma_exact_n(ctx) != 0, false, 0);
   a.qmask = (uint32_t)ctx->q - 1;
   a.B = B; a.h = h; a.h_stride = h_stride; a.r = r; a.m = m; a.value = value; a.quo = quo; a.rem = rem;
-  NTRU_IMMA_DISPATCH(k_encrypt_imma, a, NTRU_K_ENC_IMMA);
+  return for_enc_dec_form(ctx, [&](auto nj, auto limbs, auto nx) {
+    return launch_imma(ctx, k_encrypt_imma<nj, limbs, nx>, a, NTRU_K_ENC_IMMA);
+  });
 }
 
 int launch_decrypt_imma(ntru_ctx *ctx, size_t B, const int8_t *f, const uint8_t *fp, size_t key_stride, const uint16_t *e,
                         uint8_t *value, uint16_t *q1, uint16_t *r1, uint8_t *q2, uint8_t *r2) {
-  if (B == 0) return NTRU_OK;
-  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "register-fragment tensor schedule supports N <= 832");
   ImmaDecArgs a;
-  a.L = make_layout(ctx->N, imma_bucket(ctx), imma_exact_n(ctx) != 0, true);
+  a.L = make_layout(ctx->N, imma_bucket(ctx), imma_exact_n(ctx) != 0, true, 0);
   a.qmask = (uint32_t)ctx->q - 1; a.q = ctx->q; a.logq = ctx->logq;
   a.B = B; a.f = f; a.fp = fp; a.key_stride = key_stride; a.e = e;
   a.value = value; a.q1 = q1; a.r1 = r1; a.q2 = q2; a.r2 = r2;
-  NTRU_IMMA_DISPATCH(k_decrypt_imma, a, NTRU_K_DEC_IMMA);
+  return for_enc_dec_form(ctx, [&](auto nj, auto limbs, auto nx) {
+    return launch_imma(ctx, k_decrypt_imma<nj, limbs, nx>, a, NTRU_K_DEC_IMMA);
+  });
 }
 
 // ---- witness checks: the generic instantiation of each N bucket ------------------------------------------------------
-#define NTRU_CHECK_DISPATCH(KERNEL, ...)                                                                          \
-  do {                                                                                                            \
-    const int nj = a.L.NJ, wb = a.L.warp_bytes;                                                                   \
-    if (nj <= 3) return launch_imma(ctx, KERNEL<3, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                       \
-    if (nj <= 8) return launch_imma(ctx, KERNEL<8, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                       \
-    if (nj <= 11) return launch_imma(ctx, KERNEL<11, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                     \
-    return launch_imma(ctx, KERNEL<13, ##__VA_ARGS__>, a, NTRU_K_CHECK, B, wb);                                   \
-  } while (0)
-
-static int check_prologue(ntru_ctx *ctx, size_t B, CheckArgs &a, bool dec, int in_bytes, uint8_t *verdict) {
-  if (!imma_supported(ctx)) return fail(ctx, NTRU_E_UNSUPPORTED, "witness checks support N <= 832");
-  a = CheckArgs{};
-  a.L = make_check_layout(ctx->N, imma_bucket(ctx), dec, in_bytes);
+static CheckArgs check_launch_args(const ntru_ctx *ctx, size_t B, bool dec, int in_bytes, uint8_t *verdict) {
+  CheckArgs a{};
+  a.L = make_layout(ctx->N, imma_bucket(ctx), false, dec, in_bytes);
   a.M = (uint32_t)ctx->q;
   a.B = B;
   a.verdict = verdict;
-  return NTRU_OK;
+  return a;
 }
 
 int launch_check_encrypt(ntru_ctx *ctx, size_t B, const uint16_t *h, size_t h_stride, const uint8_t *r, const uint16_t *m,
                          const uint16_t *quo, const uint16_t *rem, uint8_t *verdict) {
-  if (B == 0) return NTRU_OK;
-  const size_t P = (size_t)ctx->P;
-  CheckArgs a;
-  if (int rc = check_prologue(ctx, B, a, false, 3 * ctx->P, verdict)) return rc;
-  a.x = r; a.x_stride = P; a.y = h; a.y_stride = h_stride; a.m = m; a.quo = quo; a.rem = rem;
-  NTRU_CHECK_DISPATCH(k_check_encrypt);
+  CheckArgs a = check_launch_args(ctx, B, false, 3 * ctx->P, verdict);
+  a.x = r; a.x_stride = (size_t)ctx->P; a.y = h; a.y_stride = h_stride; a.m = m; a.quo = quo; a.rem = rem;
+  return for_bucket(ctx, [&](auto nj) { return launch_imma(ctx, k_check_encrypt<nj>, a, NTRU_K_CHECK); });
 }
 
 int launch_check_decrypt(ntru_ctx *ctx, size_t B, const uint16_t *f, const uint8_t *fp, size_t key_stride, const uint16_t *e,
                          const uint16_t *q1, const uint16_t *r1, const uint8_t *q2, const uint8_t *r2, uint8_t *verdict) {
-  if (B == 0) return NTRU_OK;
-  CheckArgs a;
-  if (int rc = check_prologue(ctx, B, a, true, 5 * ctx->P, verdict)) return rc;
+  CheckArgs a = check_launch_args(ctx, B, true, 5 * ctx->P, verdict);
   a.x = f; a.fp = fp; a.x_stride = key_stride; a.y = e; a.y_stride = (size_t)ctx->P;
   a.quo = q1; a.rem = r1; a.quo2 = q2; a.rem2 = r2;
-  NTRU_CHECK_DISPATCH(k_check_decrypt);
+  return for_bucket(ctx, [&](auto nj) { return launch_imma(ctx, k_check_decrypt<nj>, a, NTRU_K_CHECK); });
 }
 
 int launch_check_inverse(ntru_ctx *ctx, size_t B, int mod_p, const uint16_t *x, const void *y, const void *quo, const void *rem,
                          uint8_t *verdict) {
-  if (B == 0) return NTRU_OK;
-  CheckArgs a;
-  if (int rc = check_prologue(ctx, B, a, false, (mod_p ? 3 : 4) * ctx->P, verdict)) return rc;
+  CheckArgs a = check_launch_args(ctx, B, false, (mod_p ? 3 : 4) * ctx->P, verdict);
   if (mod_p) a.M = (uint32_t)ctx->p;
   a.x = x; a.y = y; a.quo = quo; a.rem = rem;
-  if (mod_p) NTRU_CHECK_DISPATCH(k_check_inverse, true);
-  NTRU_CHECK_DISPATCH(k_check_inverse, false);
+  return for_bucket(ctx, [&](auto nj) {
+    return mod_p ? launch_imma(ctx, k_check_inverse<nj, true>, a, NTRU_K_CHECK) : launch_imma(ctx, k_check_inverse<nj, false>, a, NTRU_K_CHECK);
+  });
 }
 
 }  // namespace ntru

@@ -204,7 +204,7 @@ int launch_inverse(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, ui
   return NTRU_OK;
 }
 
-// fq holds f^-1 mod 2 on entry and f^-1 mod q on return; h = (p fq) * g mod (q, x^N - 1).  Rows with inverse 0 (the
+// fq holds f^-1 mod 2 on entry and f^-1 mod q on return; then h = (p fq) * g mod (q, x^N - 1).  Rows with inverse 0 (the
 // rows that are not valid) stay 0 through every step.
 int keygen_lift(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint16_t *h) {
   const int N = ctx->N, P = ctx->P;
@@ -237,14 +237,7 @@ int keygen_lift(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint1
     }
   }
   NTRU_CUDA(ctx, cudaGetLastError());
-  // h = (p fq) * g mod (q, x^N - 1): y = p fq as uint16, un-reduced (p (q - 1) < 65536; the same product modulo q as the
-  // reduced multiplyPolynomialsByScalar(fq, p, q) of index.js:75)
-  {
-    LaunchTimer timer(ctx, NTRU_K_OTHER);
-    k_scale16<<<grid, 256, 0, st>>>(fq, n, (uint32_t)ctx->p, (uint16_t *)d_t.ptr);
-  }
-  NTRU_CUDA(ctx, cudaGetLastError());
-  return launch_muldiv_imma(ctx, B, g, d_t.ptr, 0, nullptr, h);
+  return launch_h_product(ctx, B, g, fq, nullptr, h);
 }
 
 int keygen_check(ntru_ctx *ctx) {
@@ -254,6 +247,20 @@ int keygen_check(ntru_ctx *ctx) {
 }
 
 }  // namespace
+
+int launch_h_product(ntru_ctx *ctx, size_t B, const int8_t *g, const uint16_t *fq, uint16_t *quo, uint16_t *rem) {
+  // y = p fq as uint16, un-reduced (p (q - 1) < 65536; the same product modulo q as the reduced
+  // multiplyPolynomialsByScalar(fq, p, q) of index.js:75, and the y of verifyKeysInputs, index.js:155)
+  const size_t n = B * (size_t)ctx->P;
+  DevBuf &d_y = ctx->kg_bufs[0];
+  NTRU_CUDA(ctx, d_y.reserve(2 * n));
+  {
+    LaunchTimer timer(ctx, NTRU_K_OTHER);
+    k_scale16<<<(unsigned)ctx->sm_count * 8, 256, 0, ctx->stream>>>(fq, n, (uint32_t)ctx->p, (uint16_t *)d_y.ptr);
+  }
+  NTRU_CUDA(ctx, cudaGetLastError());
+  return launch_muldiv_imma(ctx, B, g, d_y.ptr, 0, quo, rem);
+}
 
 int keygen_dev(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint16_t *fq, uint8_t *fp, uint16_t *h,
                uint8_t *valid) {

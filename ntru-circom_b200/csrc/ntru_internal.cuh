@@ -63,7 +63,8 @@ struct ntru_ctx {
   ntru::DevBuf slot_bufs[ntru::kNumSlots][10];     // pitched device arrays of the host pipeline
   ntru::DevBuf slot_packed[ntru::kNumSlots][10];   // packed staging (what the 1-D H2D / D2H copies move)
   ntru::DevBuf d_partial;
-  ntru::DevBuf kg_bufs[12];         // key generation: lifting scratch (t, u0, u1, r0, r1), host-form rows, valid, count
+  ntru::DevBuf kg_bufs[12];         // key generation: lifting scratch (t, u0, u1, r0, r1), host-form rows, valid, count;
+                                    // kg_bufs[0] also holds y = p fq of launch_h_product (ntru_verify_keys_batch too)
   ntru::DevBuf check_key[2];       // witness checks, host form: the shared key row (h, or f and fp)
   ntru::DevBuf d_sum_scratch;      // tree scratch of the ciphertext sum (per-CTA rows, per-group rows, tickets)
   // cross-GPU sum: exchange window (this rank's, cudaMalloc + IPC) and the mapped windows of the peers
@@ -183,6 +184,9 @@ int keygen_batch(ntru_ctx *ctx, size_t B, const int8_t *f, const int8_t *g, uint
                  uint8_t *valid);
 int generate_keys_dev(ntru_ctx *ctx, size_t B, int df, int dg, int8_t *f, int8_t *g, uint16_t *fq, uint8_t *fp,
                       uint16_t *h);
+// h = (p fq) * g mod (q, x^N - 1) for B rows on the IMMA schedule: quotient and remainder (h) of the division by
+// 1 - x^N, either may be NULL
+int launch_h_product(ntru_ctx *ctx, size_t B, const int8_t *g, const uint16_t *fq, uint16_t *quo, uint16_t *rem);
 
 // ---- tcgen05 schedule (umma_kernels.cu) ----
 int umma_init(ntru_ctx *ctx);                    // probes the device, sets ctx->tensor_ok
